@@ -14,7 +14,8 @@ identity compaction), dynamic KV ratio 32000 / 262144 = 0.122 (keep 499 of 4096)
   cpu_baseline  the reference's own torch-op sequence (oracle/reference_ops.py) on the host cores, bounded sample
 
 --impl reference times that CPU op sequence alone (rank 0 only).  N > 1: one video per rank (weak scaling, no
-data-path collective), torchrun launch.
+data-path collective), torchrun launch.  --dump-outputs DIR writes what the last timed step computed as .npy files
+(dump_outputs()); the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -78,6 +79,8 @@ def parse():
     ap.add_argument("--no-parity", action="store_true", help="skip the kept-index parity self-check before the timed region")
     ap.add_argument("--no-sharded", action="store_true", help="N > 1: skip the within-video split record (config 3)")
     ap.add_argument("--only-sharded", action="store_true", help="N > 1: print only the within-video split record")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last timed step computed (rank 0) to DIR/<name>.npy")
     return ap.parse_args()
 
 
@@ -210,8 +213,9 @@ class ScoreTimer:
         return sum(a.elapsed_time(b) for a, b in self.pairs) / max(1, len(self.pairs)) / self.calls_per_pair
 
 
-def run_step(s, x, q, k, v, rotary, lc, vc, pos_grid, timer=None):
-    """one video through the public operators; returns a small device tensor standing for the step's result"""
+def run_step(s, x, q, k, v, rotary, lc, vc, pos_grid, timer=None, outputs=None):
+    """one video through the public operators; returns a small device tensor standing for the step's result.  A dict
+    passed as ``outputs`` receives everything the step computed: the DPSelect output and mask, and the KV cache."""
     if timer is not None and timer.on:
         a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         a.record()
@@ -247,7 +251,60 @@ def run_step(s, x, q, k, v, rotary, lc, vc, pos_grid, timer=None):
         if timer is not None and s.deferred:
             timer.arm(cache)
         cache.after_forward()                                # the chunk loop's hook (qwen2_vl.py:715-716)
+    if outputs is not None:
+        outputs.update(dpselect_out=out, dpselect_mask=mask, cache=cache)
     return cache.last_keep_indices, cache.get_seq_length(0)
+
+
+def dump_outputs(d, s, res):
+    """``res`` (run_step's ``outputs``) as ``d/<name>.npy``, float32, 64 MB at most: the DPSelect key-patch mask and
+    ``dpselect_out`` rows (of the output viewed as [t * N, C]); the compressed KV cache of every layer at a set of token
+    slots - ``kv_keys`` / ``kv_values`` [layers, KVH, slots, D], ``kv_positions`` [layers, 3 or 1, slots] with reforge -
+    and the kept indices of the last update, ``kv_last_keep_indices``.  An array larger than SAMPLE_BYTES is a fixed seeded
+    sample (sorted; its indices, float64, in ``*_rows`` / ``kv_slots``), so the files of two runs with the same arguments
+    compare element for element."""
+    import numpy as np
+    SAMPLE_BYTES = 14 << 20
+
+    def pick(n, row_bytes, seed):
+        k = max(1, SAMPLE_BYTES // row_bytes)
+        if n <= k:
+            return None
+        return torch.randperm(n, generator=torch.Generator().manual_seed(seed))[:k].sort().values
+
+    arrays = {}
+    mask = res["dpselect_mask"].reshape(-1)
+    rows = pick(mask.numel(), 4 + 8, 1)
+    if rows is not None:
+        arrays["dpselect_mask_rows"] = rows
+        mask = mask[rows.to(mask.device)]
+    arrays["dpselect_mask"] = mask
+    out = res["dpselect_out"].reshape(-1, s.C)
+    rows = pick(out.shape[0], 4 * s.C, 2)
+    if rows is not None:
+        arrays["dpselect_out_rows"] = rows
+        out = out[rows.to(out.device)]
+    arrays["dpselect_out"] = out
+    cache = res["cache"]
+    n_layers = len(cache.layers)
+    slots = pick(cache.get_seq_length(0), 8 * n_layers * s.KVH * s.D, 3)
+    if slots is None:
+        slots = torch.arange(cache.get_seq_length(0))
+    arrays["kv_slots"] = slots
+    sl = slots.to(cache.layers[0].keys.device)
+    arrays["kv_keys"] = torch.stack([cache.layers[i].keys[0].index_select(1, sl) for i in range(n_layers)])
+    arrays["kv_values"] = torch.stack([cache.layers[i].values[0].index_select(1, sl) for i in range(n_layers)])
+    if s.reforge:
+        arrays["kv_positions"] = torch.stack([cache.position_cache[i].reshape(-1, cache.position_cache[i].shape[-1])
+                                              .index_select(1, sl) for i in range(n_layers)])
+    arrays["kv_last_keep_indices"] = cache.last_keep_indices
+    arrays = {name: (t.double() if name.endswith(("_rows", "_slots")) else t.float()).cpu().numpy()
+              for name, t in arrays.items()}
+    total = sum(a_.nbytes for a_ in arrays.values())
+    assert total <= 64 << 20, f"{total} bytes of outputs"
+    os.makedirs(d, exist_ok=True)
+    for name, arr in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), arr)
 
 
 def measured_traffic(s):
@@ -664,9 +721,10 @@ def main():
     marks = []
     e0.record()
     host_s = []
-    for _ in range(a.steps):
+    last = {} if a.dump_outputs and rank == 0 else None
+    for i in range(a.steps):
         h0 = time.perf_counter()
-        res = run_step(s, x, q, k, v, rotary, lc, vc, pos_grid, timer)
+        res = run_step(s, x, q, k, v, rotary, lc, vc, pos_grid, timer, last if i == a.steps - 1 else None)
         host_s.append(time.perf_counter() - h0)          # the host's time to ENQUEUE a step (no synchronisation inside)
         marks.append(torch.cuda.Event(enable_timing=True))
         marks[-1].record()
@@ -676,6 +734,9 @@ def main():
     per_step = [p0.elapsed_time(p1) for p0, p1 in zip([e0] + marks[:-1], marks)]       # this rank's steps, device time
     launches = _native.launch_count() - launches0
     clocks = clocks_summary(sampler)
+    if last:
+        dump_outputs(a.dump_outputs, s, last)
+        del last
     ms = e0.elapsed_time(e1)
     if dist is not None:
         t = torch.tensor([ms], device=dev)

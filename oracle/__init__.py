@@ -14,7 +14,7 @@ Parity status: PINNED.  The reference has no tests or golden vectors of its
 own (SURVEY.md section 4), so the oracle is pinned against outputs of the
 *unmodified reference functions executed in the build container* (CPU torch
 2.11): ``tests/golden/make_golden.py`` imports ``/root/reference/retake`` and
-freezes its outputs into ``tests/golden/*.pt``; ``tests/test_oracle_golden.py``
+freezes its outputs into ``tests/golden/*.pt.xz``; ``tests/test_oracle_golden.py``
 replays them through this package.  The survey-time known answers KAT-D1 and
 KAT-P1 (SURVEY.md section 8c) are part of that set.
 """

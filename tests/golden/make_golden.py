@@ -12,9 +12,12 @@ It imports ``retake.visual_compression.memory_bank_compress_keyframe`` and
 ``layers[i].keys`` instead, so the reference class is instantiated through a subclass that
 only adds ``key_cache`` / ``value_cache`` list views - the reference code is not edited.
 
-Outputs: ``tests/golden/dpselect_*.pt``, ``tests/golden/pivotkv_*.pt`` and ``tests/golden/mallm_*.pt`` (inputs + outputs,
-bf16 stored as such; a few hundred KB in total).
+Outputs: ``tests/golden/dpselect_reference.pt.xz``, ``tests/golden/pivotkv_reference.pt.xz`` and
+``tests/golden/mallm_reference.pt.xz`` (inputs + outputs, bf16 stored as such; ``torch.save`` files compressed with xz,
+which removes the input rows the outputs repeat: 1.5 MB in total, each file under 1 MB; ``helpers.load_golden`` reads them).
 """
+import io
+import lzma
 import os
 import sys
 import types
@@ -25,6 +28,13 @@ REF = os.environ.get("RETAKE_REFERENCE", "/root/reference")
 HERE = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, os.path.dirname(HERE))
 from helpers import TableRotary, scene_video  # noqa: E402
+
+
+def save(cases, name):
+    buf = io.BytesIO()
+    torch.save(cases, buf)
+    with lzma.open(os.path.join(HERE, name + ".pt.xz"), "wb", preset=9 | lzma.PRESET_EXTREME) as f:
+        f.write(buf.getvalue())
 
 
 def load_reference():
@@ -106,7 +116,7 @@ def gen_dpselect(vc):
         comp, mask = vc.memory_bank_compress_keyframe(Xc, t, 3, sync=sync)
         assert torch.equal(Xc, X), "reference mutated its input"
         out.append({"name": name, "x": X, "t": t, "sync": sync, "out": comp.clone(), "mask": mask.clone()})
-    torch.save(out, os.path.join(HERE, "dpselect_reference.pt"))
+    save(out, "dpselect_reference")
     print("dpselect cases:", len(out))
 
 
@@ -176,7 +186,7 @@ def gen_pivotkv(lc):
                     "reforge": reforge, "mrope": mrope, "rotary": {"head_dim": D, "base": 10000.0,
                                                                     "attention_scaling": 1.1386},
                     "steps": steps})
-    torch.save(out, os.path.join(HERE, "pivotkv_reference.pt"))
+    save(out, "pivotkv_reference")
     print("pivotkv cases:", len(out))
 
 
@@ -200,7 +210,7 @@ def gen_mallm(vc):
             keep = [0, len(rounds) // 2, len(rounds) - 1]                # first / middle / last round only (file size)
             out.append({"name": name, "x": X, "t": t, "sync": sync, "n_rounds": len(rounds),
                         "rounds": {i: rounds[i] for i in keep}})
-    torch.save(out, os.path.join(HERE, "mallm_reference.pt"))
+    save(out, "mallm_reference")
     print("mallm cases:", len(out))
 
 

@@ -1,5 +1,15 @@
 """Shared synthetic-input helpers for tests, golden generation and bench (no reference, no oracle)."""
+import io
+import lzma
+import os
+
 import torch
+
+
+def load_golden(name):
+    """the cases frozen by tests/golden/make_golden.py: ``tests/golden/<name>.pt.xz``, an xz-compressed ``torch.save`` file"""
+    with lzma.open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", name + ".pt.xz")) as f:
+        return torch.load(io.BytesIO(f.read()))
 
 
 class TableRotary:

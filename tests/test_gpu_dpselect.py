@@ -1,16 +1,14 @@
 """GPU parity: DPSelect kernels (through the C ABI) against the oracle and against the reference's own
 torch-op sequence executed on the same B200 (the bit-exactness target, SURVEY.md 8a note N4)."""
-import os
 
 import pytest
 import torch
 import torch.nn.functional as F
 
-from helpers import scene_video
+from helpers import load_golden, scene_video
 from oracle import dpselect as od
 
 pytestmark = pytest.mark.gpu
-G = os.path.join(os.path.dirname(__file__), "golden")
 
 
 def _mods():
@@ -140,7 +138,7 @@ def test_operator_matches_reference_ops_on_cuda(kind, T, N, C, seed, sync):
 def test_golden_fixtures_through_cuda():
     """frozen CPU-reference outputs: equal whenever the CUDA-order distances tie-freely agree"""
     vc = _mods()
-    cases = torch.load(os.path.join(G, "dpselect_reference.pt"))
+    cases = load_golden("dpselect_reference")
     ran = 0
     for c in cases:
         x = c["x"]

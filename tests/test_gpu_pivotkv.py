@@ -1,17 +1,15 @@
 """GPU parity: PivotKV kernels (through the C ABI) against the oracle and against the reference's own
 torch-op sequence executed on the same B200."""
 import math
-import os
 import types
 
 import pytest
 import torch
 
-from helpers import TableRotary
+from helpers import TableRotary, load_golden
 from oracle import pivotkv as op
 
 pytestmark = pytest.mark.gpu
-G = os.path.join(os.path.dirname(__file__), "golden")
 BF = torch.bfloat16
 
 
@@ -192,7 +190,7 @@ def test_update_replays_golden_steps_bf16():
     """frozen reference runs (CPU, bf16) replayed through the CUDA cache: shapes, bookkeeping, values as gathers,
     kept sets tie/ulp-aware against the oracle's CUDA-semantics scores."""
     lc = _lc()
-    cases = [c for c in torch.load(os.path.join(G, "pivotkv_reference.pt"))
+    cases = [c for c in load_golden("pivotkv_reference")
              if c["name"] in ("chunks_bf16_reforge", "chunks_bf16_noreforge")]
     assert len(cases) == 2
     for case in cases:

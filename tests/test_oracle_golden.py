@@ -4,18 +4,16 @@ CPU only.  ``tie="torch"`` replays ``torch.topk`` on the same device the referen
 everything must be bit-identical; ``tie="lowest"`` (the CUDA rule the kernels implement) must agree
 wherever the selection boundary is tie-free and be tie-consistent otherwise.
 """
-import os
 
 import pytest
 import torch
 
-from helpers import TableRotary
+from helpers import TableRotary, load_golden
 from oracle import dpselect as od
 from oracle import pivotkv as op
 
-G = os.path.join(os.path.dirname(__file__), "golden")
-DP = torch.load(os.path.join(G, "dpselect_reference.pt"))
-PK = torch.load(os.path.join(G, "pivotkv_reference.pt"))
+DP = load_golden("dpselect_reference")
+PK = load_golden("pivotkv_reference")
 
 
 def _id(c):
@@ -207,7 +205,7 @@ def test_reference_ops_pivot_update_bit_identical(case):
 # ------------------------------------------------------------------------------------------- MA-LLM compressors
 from oracle import mallm as om  # noqa: E402
 
-ML = torch.load(os.path.join(G, "mallm_reference.pt"))
+ML = load_golden("mallm_reference")
 
 
 def _replay_mallm(case, soft_round, hard_round):
