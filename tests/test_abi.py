@@ -45,6 +45,14 @@ def test_argument_errors_without_gpu():
     assert lib.rtk_pivot_score_workspace_bytes(28, 4096) == 10 * 28 * 4096 * 4
     assert lib.rtk_pivot_score_workspace_bytes(4, 130) == 10 * 4 * 256 * 4
     assert lib.rtk_pivot_select(a16, 4, 16, None, 17, a16, None, None) == -1   # keep > L
+    # one step outside the documented limits: RTK_E_UNSUPPORTED before any CUDA call
+    assert lib.rtk_dpselect_select(a16, 8193, 4, 9, 0, a16, a16, None) == -3   # T <= 8192
+    assert lib.rtk_dpselect_select(a16, 8193, 4, 9, 1, a16, a16, None) == -3
+    for T, N, C in ((8193, 4, 256), (4, 65536, 256), (4, 4, 8200)):            # T <= 8192, N <= 65535, C <= 8192
+        assert lib.rtk_mallm_compress(a16, None, T, N, C, 2, 0, 0, a16, a16, a16, 1 << 40, None) == -3, (T, N, C)
+    assert lib.rtk_pivot_score(a16, 4, 128, 512, a16, 2, 128, 256, 16385, 128, a16, a16, 1 << 40, None) == -3  # L
+    assert lib.rtk_pivot_score(a16, 264, 128, 512, a16, 8, 128, 256, 16, 128, a16, a16, 1 << 40, None) == -3  # H <= 256
+    assert lib.rtk_pivot_select(a16, 4, 16385, None, 17, a16, None, None) == -3    # L <= 16384
     # batched update: workspace query, argument errors
     one = lib.rtk_pivot_update_batch_workspace_bytes(28, 4, 4096, 128, 1)
     assert lib.rtk_pivot_update_batch_workspace_bytes(28, 4, 4096, 128, 28) > 27 * (one - 1024) > 0

@@ -70,6 +70,7 @@ SHAPES = [  # H, KVH, L, D, layers, chunks, ratio, reforge, mrope
     (8, 2, 200, 128, 2, 2, 0.3, True, None),
     (28, 4, 1024, 128, 4, 2, 0.122, True, [16, 24, 24]),
     (28, 4, 1024, 128, 3, 2, 0.5, False, [16, 24, 24]),
+    (28, 4, 16384, 128, 4, 1, 0.25, True, [16, 24, 24]),       # the length limit, 4 layers in one batched call
 ]
 
 

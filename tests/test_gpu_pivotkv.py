@@ -28,8 +28,12 @@ def qkv(H, KVH, L, D, alpha, seed, transposed=True):
 
 
 def ref_head_scores_cuda(q, k):
-    """longvideo_cache.py:260-269 with stock ATen/cuBLAS ops on the GPU (the reference as it runs on CUDA)."""
+    """longvideo_cache.py:260-269 with stock ATen/cuBLAS ops on the GPU (the reference as it runs on CUDA).  Beyond
+    L = 6272 the [H, L, L] logits of one call would take tens of GB: there one KV-head group is scored at a time."""
     H, KVH, L, D = q.shape[1], k.shape[1], q.shape[2], q.shape[3]
+    if L > 6272 and KVH > 1:
+        G = H // KVH
+        return torch.cat([ref_head_scores_cuda(q[:, g * G:(g + 1) * G], k[:, g:g + 1]) for g in range(KVH)])
     kr = k[:, :, None].expand(1, KVH, H // KVH, L, D).reshape(1, H, L, D)
     w = torch.matmul(q, kr.transpose(2, 3)) / math.sqrt(D)
     w = torch.nn.functional.softmax(w, dim=-1, dtype=torch.float32).to(q.dtype)
@@ -46,7 +50,10 @@ def ulp_diff(a, b):
 
 SCORE_SHAPES = [(4, 2, 128, 64, 1.0), (4, 2, 1024, 64, 1.0), (14, 2, 96, 64, 3.0), (28, 4, 256, 128, 1.0),
                 (28, 4, 1000, 128, 3.0), (8, 8, 130, 128, 1.0), (28, 4, 4096, 128, 1.0), (4, 1, 1, 128, 1.0),
-                (28, 4, 2304, 128, 3.0)]
+                (28, 4, 2304, 128, 3.0),
+                # the length and head limits (rtk_b200.h): 12289 = 96 full tiles and one ragged one, H = 256
+                (28, 4, 8192, 128, 1.0), (28, 4, 12289, 128, 1.0), (28, 4, 16384, 128, 1.0), (16, 2, 16384, 64, 1.0),
+                (256, 32, 1024, 128, 1.0)]
 
 
 @pytest.mark.parametrize("H,KVH,L,D,alpha", SCORE_SHAPES)
@@ -84,7 +91,7 @@ def test_head_scores_layout_independent():
 
 
 @pytest.mark.parametrize("L,keep", [(16, 8), (1024, 512), (4096, 1024), (4096, 499), (6272, 1568), (2304, 2304),
-                                    (1, 1), (130, 1)])
+                                    (1, 1), (130, 1), (16384, 4096), (16384, 16384), (16383, 1)])
 def test_select_bit_exact_vs_torch_on_cuda(L, keep):
     lc = _lc()
     g = torch.Generator().manual_seed(L + keep)

@@ -508,11 +508,17 @@ extern "C" int rtk_dpselect_select(const float* dis, int64_t T, int64_t N, int64
         if (e != cudaSuccess) return (int)e;
         dpselect_select_sync_kernel<<<1, kSyncWarps * kWarp, smem, st>>>(dis, (int)T, (int)N, (int)t, idx, mask);
     } else {
+        int dev = 0, smem_max = 0;
+        cudaGetDevice(&dev);
+        cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
         int W = kSelWarps;                                      // patches per CTA: fewer when that still leaves >= ~2 CTAs per SM
         while (W > 1 && (N + W - 1) / W < 296) W >>= 1;
+        // and fewer when W columns of T distances + peak flags do not fit (8 columns stop fitting at T = 5812 on a B200;
+        // one warp per column, so W does not change the result)
+        while (W > 1 && (size_t)W * T * 5 > (size_t)smem_max) W >>= 1;
         const size_t smem = (size_t)W * T * 5;
         cudaError_t e = cudaFuncSetAttribute(dpselect_select_patch_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                             (int)((size_t)kSelWarps * T * 5));
+                                             (int)smem);
         if (e != cudaSuccess) return (int)e;
         const unsigned grid = (unsigned)((N + W - 1) / W);
         dpselect_select_patch_kernel<<<grid, W * kWarp, smem, st>>>(dis, (int)T, (int)N, (int)t, idx, mask);

@@ -793,7 +793,8 @@ extern "C" int rtk_mallm_compress(const void* x, const void* sizes_in, int64_t T
                 if (e2 != cudaSuccess) return (int)e2;
                 RTK_LAUNCH_PDL(mallm_rounds_smem_kernel, (unsigned)N, kMlThreads, need, stream, P, rounds);
             } else {                                              // very long videos: state stays in global memory
-                RTK_LAUNCH_PDL(mallm_rounds_kernel, (unsigned)N, kMlThreads, scan_smem, stream, P, rounds);
+                // only the similarity column lives in shared memory: T floats, at most 32 KB, under the 48 KB default
+                RTK_LAUNCH_PDL(mallm_rounds_kernel, (unsigned)N, kMlThreads, (size_t)T * 4, stream, P, rounds);
             }
         }
     } else {
