@@ -239,16 +239,20 @@ typedef struct rtk_pivot_update_args {
     uint32_t* xchg_flags[8];
 } rtk_pivot_update_args;
 
+/* == rtk_pivot_update_batch_workspace_bytes(H, KVH, L, D, 1) */
 size_t rtk_pivot_update_workspace_bytes(int64_t H, int64_t KVH, int64_t L, int64_t D);
-/* With inv_freq the kept keys come back re-rotated; with cos/sin tables (opaque rotary callable) the caller
- * finishes with rotary_emb_fn(v_out, pos_out) + rtk_pivot_rope(forward=1). */
+/* rtk_pivot_update_batch for one layer: the same launches, workspace layout and argument checks, all of which come before
+ * the first launch (a call with skip_select or skip_score is not checked for what only the skipped step reads).  With
+ * inv_freq the kept keys come back re-rotated; with cos/sin tables (opaque rotary callable) the caller finishes with
+ * rotary_emb_fn(v_out, pos_out) + rtk_pivot_rope(forward=1). */
 int rtk_pivot_update(const rtk_pivot_update_args* args, void* stream);
 
 /* The compressing updates of ALL layers of one chunk in one chain of seven launches (deferred compression: the
  * reference's chunk loop calls past_key_values.after_forward() once the chunk's forward is done, retake/qwen2_vl.py:715-716,
  * and a chunk's kept rows are first needed by the NEXT chunk - SURVEY.md 8(f2)).  layers[i] describes layer i exactly as
  * for rtk_pivot_update; H, KVH, L, D, keep, reforge, n_pos, mrope_section and the rotary (inv_freq, attention_scaling)
- * must be the same for every layer, reforge needs inv_freq (RTK_E_UNSUPPORTED otherwise: use rtk_pivot_update), pointers
+ * must be the same for every layer, reforge with cos/sin tables instead of inv_freq takes one layer (RTK_E_UNSUPPORTED
+ * otherwise: one rtk_pivot_update per layer), pointers
  * and strides are per layer; k_out / v_out may point straight into the layer's cache (rows D apart, heads out_stride_h
  * apart) and pos_out into its position cache (rows pos_out_stride apart).  layers[i].workspace is ignored; `workspace`
  * (256-byte aligned) holds the un-rotated Q / K copies and the row statistics of min(n_layers, 32) layers - more layers

@@ -57,6 +57,7 @@ def test_argument_errors_without_gpu():
     one = lib.rtk_pivot_update_batch_workspace_bytes(28, 4, 4096, 128, 1)
     assert lib.rtk_pivot_update_batch_workspace_bytes(28, 4, 4096, 128, 28) > 27 * (one - 1024) > 0
     assert lib.rtk_pivot_update_batch_workspace_bytes(28, 4, 4096, 128, 64) == lib.rtk_pivot_update_batch_workspace_bytes(28, 4, 4096, 128, 32)
+    assert lib.rtk_pivot_update_workspace_bytes(28, 4, 4096, 128) >= one       # rtk_pivot_update runs a one-layer batch
     assert lib.rtk_pivot_update_batch(None, 2, a16, 1 << 20, None) == -1
     from retake.longvideo_cache import _UpdateArgs
     arr = (_UpdateArgs * 2)()

@@ -21,6 +21,16 @@ struct RopeParams {
     float inv_scale2;
 };
 
+// RopeParams::bound from the mrope sections (all zero unless n_pos == 3); false when 3-D sections do not cover D
+static bool mrope_bounds(int n_pos, const int32_t* sec, int64_t D, int bound[6]) {
+    int acc = 0;
+    for (int i = 0; i < 6; ++i) {
+        acc += n_pos == 3 ? sec[i % 3] : 0;
+        bound[i] = acc;
+    }
+    return n_pos != 3 || acc == D;
+}
+
 __device__ __forceinline__ int rope_pos_row(const RopeParams& p, int c) {
     if (p.n_pos == 1) return 0;
     int i = 0;
@@ -181,15 +191,8 @@ __device__ __forceinline__ void unrope_qk_body(const __nv_bfloat16* __restrict__
     }
 }
 
-__global__ void __launch_bounds__(256)
-pivot_unrope_qk_kernel(const __nv_bfloat16* __restrict__ x, const long long* __restrict__ pos, const float* __restrict__ inv_freq,
-                       float scaling, __nv_bfloat16* __restrict__ out, RopeParams p) {
-    pdl_enter();
-    unrope_qk_body(x, pos, inv_freq, scaling, out, p);
-}
-
-// Per-layer tables of a batched update (rtk_pivot_update_batch): every layer of the chunk brings its own tensors, the
-// shapes are shared.  Passed as ONE __grid_constant__ kernel parameter (4.9 KB).
+// Per-layer tables of an update (rtk_pivot_update_batch; rtk_pivot_update is a batch of one): every layer of the chunk
+// brings its own tensors, the shapes are shared.  Passed as ONE __grid_constant__ kernel parameter (4.9 KB).
 struct BatchLayers {
     const __nv_bfloat16* q[kMaxBatchLayers];         // caller's views (un-rotation input)
     const __nv_bfloat16* k[kMaxBatchLayers];         // K the compaction reads (the un-rotated copy when re-forging)
@@ -502,35 +505,8 @@ __device__ __forceinline__ void xchg_wait(const uint32_t* flags, int n, uint32_t
     }
     __syncthreads();
 }
-struct XchgPut {
-    const __nv_bfloat16* src;        // this rank's rows inside its own buffer
-    __nv_bfloat16* dst[8];           // the same rows inside every rank's buffer (dst[rank] == src: skipped)
-    uint32_t* flags[8];              // flags[r] + rank is written with the epoch
-    long long n;                     // bf16 elements
-    int world, rank;
-    uint32_t epoch;
-};
-__global__ void __launch_bounds__(1024)
-pivot_xchg_put_kernel(XchgPut p) {
-    pdl_enter();
-    for (int r = 0; r < p.world; ++r) {
-        if (r == p.rank) continue;
-        __nv_bfloat16* dst = p.dst[r];
-        if ((((uintptr_t)p.src | (uintptr_t)dst) & 15u) == 0) {
-            const long long nv = p.n >> 3;
-            for (long long i = threadIdx.x; i < nv; i += blockDim.x)
-                reinterpret_cast<uint4*>(dst)[i] = reinterpret_cast<const uint4*>(p.src)[i];
-            for (long long i = (nv << 3) + threadIdx.x; i < p.n; i += blockDim.x) dst[i] = p.src[i];
-        } else {
-            for (long long i = threadIdx.x; i < p.n; i += blockDim.x) dst[i] = p.src[i];
-        }
-    }
-    __threadfence_system();          // every thread's peer stores are performed before ...
-    __syncthreads();
-    if ((int)threadIdx.x < p.world) st_release_sys(p.flags[threadIdx.x] + p.rank, p.epoch);      // ... the flags go up
-}
-
-// the same for all layers of a chunk: one CTA per layer moves that layer's rows, a one-CTA kernel behind it raises the flags
+// one CTA per layer of the chunk stores this rank's rows into every peer's buffer (dst[layer][rank]: skipped), a one-CTA
+// kernel behind it raises the flags
 struct XchgPutBatch {
     const __nv_bfloat16* src[kMaxBatchLayers];
     __nv_bfloat16* dst[kMaxBatchLayers][8];
@@ -570,13 +546,9 @@ pivot_xchg_flag_kernel(XchgFlags p) {
 
 __global__ void __launch_bounds__(kSelThreads)
 pivot_select_kernel(const __nv_bfloat16* __restrict__ head_scores, int KVH, int L, const uint8_t* __restrict__ keymask,
-                    int keep, int32_t* __restrict__ keep_idx, __nv_bfloat16* __restrict__ score_out,
-                    const long long* __restrict__ tpos, long long* __restrict__ tmin_out,
-                    const uint32_t* __restrict__ wait_flags, int wait_n, uint32_t wait_epoch, unsigned long long wait_ns) {
+                    int keep, int32_t* __restrict__ keep_idx, __nv_bfloat16* __restrict__ score_out) {
     pdl_enter();
-    // rows of the other ranks arrive over NVLink: nothing of head_scores is read before every rank's flag is up
-    if (wait_flags) xchg_wait(wait_flags, wait_n, wait_epoch, wait_ns);
-    pivot_select_body(head_scores, KVH, L, keymask, keep, keep_idx, score_out, tpos, tmin_out);
+    pivot_select_body(head_scores, KVH, L, keymask, keep, keep_idx, score_out, nullptr, nullptr);
 }
 
 // one CTA per layer of the chunk
@@ -584,6 +556,7 @@ __global__ void __launch_bounds__(kSelThreads)
 pivot_select_batch_kernel(const __grid_constant__ BatchLayers t, int KVH, int L, int keep, int reforge, long long* __restrict__ tmin,
                           const uint32_t* __restrict__ wait_flags, int wait_n, uint32_t wait_epoch, unsigned long long wait_ns) {
     pdl_enter();
+    // rows of the other ranks arrive over NVLink: nothing of head_scores is read before every rank's flag is up
     if (wait_flags) xchg_wait(wait_flags, wait_n, wait_epoch, wait_ns);
     const int layer = blockIdx.x;
     pivot_select_body(t.head_scores[layer], KVH, L, t.keymask[layer], keep, t.keep_idx[layer], nullptr,
@@ -704,16 +677,6 @@ __device__ __forceinline__ void compact_rope_body(const __nv_bfloat16* __restric
     }
 }
 
-__global__ void __launch_bounds__(128)
-pivot_compact_rope_kernel(const __nv_bfloat16* __restrict__ k, const __nv_bfloat16* __restrict__ v,
-                          const int32_t* __restrict__ keep_idx, __nv_bfloat16* __restrict__ k_out,
-                          __nv_bfloat16* __restrict__ v_out, const long long* __restrict__ pos, long long* __restrict__ pos_out,
-                          const long long* __restrict__ tmin, const float* __restrict__ inv_freq, float scaling, CompactParams p,
-                          RopeParams rp, int rotate) {
-    pdl_enter();
-    compact_rope_body(k, v, keep_idx, k_out, v_out, pos, pos_out, tmin, inv_freq, scaling, p, rp, rotate);
-}
-
 // grid (keep, layers): kept rows of every layer of the chunk straight into their caches
 __global__ void __launch_bounds__(128)
 pivot_compact_rope_batch_kernel(const __grid_constant__ BatchLayers t, const long long* __restrict__ tmin,
@@ -818,6 +781,15 @@ extern "C" const char* rtk_error_string(int code) {
     }
 }
 
+// pivot_rope_kernel over the p.heads rows of x and the p.heads2 rows of p.x2
+static int rope_launch(const void* x, const void* cos, const void* sin, void* out, const RopeParams& p, cudaStream_t st) {
+    const long long total = (long long)(p.heads + p.heads2) * p.L * (p.D / 16);
+    long long grid = (total + 255) / 256;
+    if (grid > 148 * 16) grid = 148 * 16;
+    RTK_LAUNCH_PDL(pivot_rope_kernel, (unsigned)grid, 256, 0, st, (const __nv_bfloat16*)x, (const __nv_bfloat16*)cos, (const __nv_bfloat16*)sin, (__nv_bfloat16*)out, p);
+    return 0;
+}
+
 extern "C" int rtk_pivot_rope(const void* x, int64_t heads, int64_t L, int64_t D, int64_t stride_h, int64_t stride_l,
                               const void* cos, const void* sin, int n_pos, const int32_t* mrope_section_host,
                               float inv_scale2, int forward, void* out, int64_t out_stride_h, int64_t out_stride_l,
@@ -834,17 +806,8 @@ extern "C" int rtk_pivot_rope(const void* x, int64_t heads, int64_t L, int64_t D
     p.inv_scale2 = inv_scale2;
     p.heads2 = 0; p.x2 = nullptr; p.out2 = nullptr;
     p.stride_h2 = p.stride_l2 = p.out_stride_h2 = p.out_stride_l2 = 0;
-    int acc = 0;
-    for (int i = 0; i < 6; ++i) {
-        acc += (n_pos == 3) ? mrope_section_host[i % 3] : 0;
-        p.bound[i] = acc;
-    }
-    if (n_pos == 3 && acc != D) return RTK_E_UNSUPPORTED;
-    const long long total = heads * L * (D / 16);
-    long long grid = (total + 255) / 256;
-    if (grid > 148 * 16) grid = 148 * 16;
-    RTK_LAUNCH_PDL(pivot_rope_kernel, (unsigned)grid, 256, 0, (cudaStream_t)stream,  (const __nv_bfloat16*)x, (const __nv_bfloat16*)cos, (const __nv_bfloat16*)sin, (__nv_bfloat16*)out, p);
-    return 0;
+    if (!mrope_bounds(n_pos, mrope_section_host, D, p.bound)) return RTK_E_UNSUPPORTED;
+    return rope_launch(x, cos, sin, out, p, (cudaStream_t)stream);
 }
 
 extern "C" int rtk_pivot_select(const void* head_scores, int64_t KVH, int64_t L, const uint8_t* keymask, int64_t keep,
@@ -856,37 +819,25 @@ extern "C" int rtk_pivot_select(const void* head_scores, int64_t KVH, int64_t L,
     cudaError_t e = cudaFuncSetAttribute(pivot_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
     if (e != cudaSuccess) return (int)e;
     RTK_LAUNCH_PDL(pivot_select_kernel, 1, kSelThreads, smem, (cudaStream_t)stream, (const __nv_bfloat16*)head_scores, (int)KVH,
-                   (int)L, keymask, (int)keep, keep_idx, (__nv_bfloat16*)score_out, (const long long*)nullptr, (long long*)nullptr,
-                   (const uint32_t*)nullptr, 0, 0u, 0ull);
+                   (int)L, keymask, (int)keep, keep_idx, (__nv_bfloat16*)score_out);
     return 0;
 }
-
-static int compact_kv(const void* k, const void* v, int64_t KVH, int64_t L, int64_t D, int64_t stride_h, int64_t stride_l,
-                      int64_t v_stride_h, int64_t v_stride_l, const int32_t* keep_idx, int64_t keep, void* k_out, void* v_out,
-                      int64_t out_stride_h, const int64_t* pos, int n_pos, int64_t* pos_out, int reforge, void* stream);
 
 extern "C" int rtk_pivot_compact(const void* k, const void* v, int64_t KVH, int64_t L, int64_t D, int64_t stride_h,
                                  int64_t stride_l, const int32_t* keep_idx, int64_t keep, void* k_out, void* v_out,
                                  int64_t out_stride_h, const int64_t* pos, int n_pos, int64_t* pos_out, int reforge,
                                  void* stream) {
     RTK_NVTX("rtk_pivot_compact");
-    return compact_kv(k, v, KVH, L, D, stride_h, stride_l, stride_h, stride_l, keep_idx, keep, k_out, v_out, out_stride_h, pos,
-                      n_pos, pos_out, reforge, stream);
-}
-
-static int compact_kv(const void* k, const void* v, int64_t KVH, int64_t L, int64_t D, int64_t stride_h, int64_t stride_l,
-                      int64_t v_stride_h, int64_t v_stride_l, const int32_t* keep_idx, int64_t keep, void* k_out, void* v_out,
-                      int64_t out_stride_h, const int64_t* pos, int n_pos, int64_t* pos_out, int reforge, void* stream) {
     if ((!k && !v) || !keep_idx || (k && !k_out) || (v && !v_out) || KVH < 1 || L < 1 || D < 8 || keep < 1 || keep > L)
         return RTK_E_BADARG;
     if (pos && (!pos_out || n_pos < 1)) return RTK_E_BADARG;
     if (D % 8 != 0) return RTK_E_UNSUPPORTED;
     if ((((uintptr_t)k | (uintptr_t)v | (uintptr_t)k_out | (uintptr_t)v_out) & 15u) != 0) return RTK_E_ALIGN;   // NULL passes
-    if ((stride_h | stride_l | v_stride_h | v_stride_l | out_stride_h) % 8 != 0) return RTK_E_ALIGN;
+    if ((stride_h | stride_l | out_stride_h) % 8 != 0) return RTK_E_ALIGN;
     CompactParams p;
     p.KVH = (int)KVH; p.L = (int)L; p.D = (int)D; p.keep = (int)keep; p.n_pos = n_pos; p.reforge = reforge;
     p.stride_h = stride_h; p.stride_l = stride_l; p.out_stride_h = out_stride_h;
-    p.v_stride_h = v_stride_h; p.v_stride_l = v_stride_l;
+    p.v_stride_h = stride_h; p.v_stride_l = stride_l;
     p.pos_out_stride = keep;
     p.ratio = (float)((double)keep / (double)L);
     const long long total = KVH * keep * (D / 8);
@@ -909,196 +860,14 @@ extern "C" int rtk_pivot_rope_tables(const int64_t* pos, int n_pos, int64_t L, i
     p.heads2 = 0; p.x2 = nullptr; p.out2 = nullptr;
     p.stride_h2 = p.stride_l2 = p.out_stride_h2 = p.out_stride_l2 = 0;
     p.inv_scale2 = 1.0f;
-    int acc = 0;
-    for (int i = 0; i < 6; ++i) {
-        acc += (n_pos == 3) ? mrope_section_host[i % 3] : 0;
-        p.bound[i] = acc;
-    }
-    if (n_pos == 3 && acc != D) return RTK_E_UNSUPPORTED;
+    if (!mrope_bounds(n_pos, mrope_section_host, D, p.bound)) return RTK_E_UNSUPPORTED;
     long long grid = (L * D + 255) / 256;
     if (grid > 148 * 8) grid = 148 * 8;
     RTK_LAUNCH_PDL(pivot_rope_table_kernel, (unsigned)grid, 256, 0, (cudaStream_t)stream,  (const long long*)pos, inv_freq, p, attention_scaling, (__nv_bfloat16*)cos_out, (__nv_bfloat16*)sin_out);
     return 0;
 }
 
-// un-rotate q and k with pre-selected [L, D] tables in ONE launch
-static int rope_qk_reverse(const void* q, int64_t H, int64_t qsh, int64_t qsl, const void* k, int64_t KVH, int64_t ksh, int64_t ksl,
-                           int64_t L, int64_t D, const void* cos, const void* sin, int n_pos, const int32_t* sec, float inv_scale2,
-                           void* qu, void* ku, cudaStream_t st) {
-    if ((((uintptr_t)q | (uintptr_t)k | (uintptr_t)qu | (uintptr_t)ku) & 15u) != 0) return RTK_E_ALIGN;
-    if ((qsh | qsl | ksh | ksl) % 8 != 0 || D % 16 != 0) return RTK_E_ALIGN;
-    RopeParams p;
-    p.heads = (int)H; p.L = (int)L; p.D = (int)D; p.n_pos = n_pos; p.forward = 0;
-    p.stride_h = qsh; p.stride_l = qsl; p.out_stride_h = L * D; p.out_stride_l = D;
-    p.heads2 = (int)KVH; p.x2 = (const __nv_bfloat16*)k; p.out2 = (__nv_bfloat16*)ku;
-    p.stride_h2 = ksh; p.stride_l2 = ksl; p.out_stride_h2 = L * D; p.out_stride_l2 = D;
-    p.inv_scale2 = inv_scale2;
-    int acc = 0;
-    for (int i = 0; i < 6; ++i) {
-        acc += (n_pos == 3 && sec) ? sec[i % 3] : 0;
-        p.bound[i] = acc;
-    }
-    if (n_pos == 3 && acc != D) return RTK_E_UNSUPPORTED;
-    const long long total = (H + KVH) * L * (D / 16);
-    long long grid = (total + 255) / 256;
-    if (grid > 148 * 16) grid = 148 * 16;
-    RTK_LAUNCH_PDL(pivot_rope_kernel, (unsigned)grid, 256, 0, st, (const __nv_bfloat16*)q, (const __nv_bfloat16*)cos, (const __nv_bfloat16*)sin, (__nv_bfloat16*)qu, p);
-    return 0;
-}
-
 static size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
-
-extern "C" size_t rtk_pivot_update_workspace_bytes(int64_t H, int64_t KVH, int64_t L, int64_t D) {
-    if (H < 1 || KVH < 1 || L < 1 || D < 1) return 0;
-    return align256(rtk_pivot_score_workspace_bytes(H, L)) + align256((size_t)H * L * D * 2) + align256((size_t)KVH * L * D * 2) +
-           4 * align256((size_t)L * D * 2) + 256 + key_elide_bytes(KVH, L, D) + 256;
-}
-
-extern "C" int rtk_pivot_update(const rtk_pivot_update_args* a, void* stream) {
-    RTK_NVTX("rtk_pivot_update");
-    if (!a || !a->q || !a->k || !a->v || !a->k_out || !a->v_out || !a->keep_idx || !a->head_scores || !a->workspace)
-        return RTK_E_BADARG;
-    if (a->workspace_bytes < rtk_pivot_update_workspace_bytes(a->H, a->KVH, a->L, a->D)) return RTK_E_WORKSPACE;
-    if (((uintptr_t)a->workspace & 255u) != 0) return RTK_E_ALIGN;
-    const int64_t H = a->H, KVH = a->KVH, L = a->L, D = a->D;
-    char* ws = (char*)a->workspace;
-    void* score_ws = ws;                ws += align256(rtk_pivot_score_workspace_bytes(H, L));
-    void* qu = ws;                      ws += align256((size_t)H * L * D * 2);
-    void* ku = ws;                      ws += align256((size_t)KVH * L * D * 2);
-    void* cos1 = ws;                    ws += align256((size_t)L * D * 2);
-    void* sin1 = ws;                    ws += align256((size_t)L * D * 2);
-    void* cos2 = ws;                    ws += align256((size_t)L * D * 2);
-    void* sin2 = ws;                    ws += align256((size_t)L * D * 2);
-    long long* tmin = (long long*)ws;    ws += 256;   // smallest kept temporal position (select -> fused compaction)
-    char* kc_ws = ws;                    ws += align256((size_t)KVH * L * D * 2);      // key elision: compact K copy,
-    int32_t* slot_ws = (int32_t*)ws;     ws += align256((size_t)L * 4);                //   slots,
-    int32_t* nkeys_ws = (int32_t*)ws;                                                   //   count
-    (void)cos2; (void)sin2;
-    const void* q = a->q;
-    const void* k = a->k;
-    int64_t qsh = a->q_stride_h, qsl = a->q_stride_l, ksh = a->k_stride_h, ksl = a->k_stride_l;
-    int rc;
-    const bool fused_tables = a->reforge && a->inv_freq;
-    const bool xchg = a->xchg_world > 1;
-    if (a->skip_score && a->skip_select) return RTK_E_BADARG;
-    if (xchg) {
-        if (a->xchg_world > 8 || a->xchg_rank < 0 || a->xchg_rank >= a->xchg_world || !(a->skip_select || a->skip_score))
-            return RTK_E_BADARG;
-        for (int r = 0; r < a->xchg_world; ++r)
-            if (!a->xchg_scores[r] || !a->xchg_flags[r]) return RTK_E_BADARG;
-        // where the rows live is part of the protocol: checked before anything is launched
-        const char* own = (const char*)a->xchg_scores[a->xchg_rank];
-        if (a->skip_select && (const char*)a->head_scores != own + (size_t)a->xchg_rank * KVH * L * 2) return RTK_E_BADARG;
-        if (a->skip_score && (const char*)a->head_scores != own) return RTK_E_BADARG;
-    }
-    const int64_t score_rows = a->score_rows > 0 ? a->score_rows : KVH;
-    if (a->reforge) {
-        if (!a->pos || !a->pos_out) return RTK_E_BADARG;
-        const void *c = a->cos, *s = a->sin;
-        int n_pos_tab = a->n_pos;
-        const int32_t* sec = a->n_pos == 3 ? a->mrope_section : nullptr;
-        if (fused_tables) {
-            // tables computed inside the rotation kernel: one launch for q and k
-            if ((((uintptr_t)q | (uintptr_t)k) & 15u) != 0 || (qsh | qsl | ksh | ksl) % 8 != 0 || D % 16 != 0 || D > 256) return RTK_E_ALIGN;
-            RopeParams p;
-            p.heads = (int)H; p.L = (int)L; p.D = (int)D; p.n_pos = a->n_pos; p.forward = 0;
-            p.stride_h = qsh; p.stride_l = qsl; p.out_stride_h = L * D; p.out_stride_l = D;
-            p.heads2 = (int)KVH; p.x2 = (const __nv_bfloat16*)k; p.out2 = (__nv_bfloat16*)ku;
-            p.stride_h2 = ksh; p.stride_l2 = ksl; p.out_stride_h2 = L * D; p.out_stride_l2 = D;
-            p.inv_scale2 = a->inv_scale2;
-            int acc = 0;
-            for (int i = 0; i < 6; ++i) {
-                acc += sec ? sec[i % 3] : 0;
-                p.bound[i] = acc;
-            }
-            if (sec && acc != D) return RTK_E_UNSUPPORTED;
-            // (skip_score: the copies of the preceding skip_select call are still in the workspace)
-            if (!a->skip_score)
-                RTK_LAUNCH_PDL(pivot_unrope_qk_kernel, (unsigned)((L + kUnropeTok - 1) / kUnropeTok), 256, 0, (cudaStream_t)stream, (const __nv_bfloat16*)q,
-                               (const long long*)a->pos, a->inv_freq, a->attention_scaling, (__nv_bfloat16*)qu, p);
-        } else {
-            if (!c || !s) return RTK_E_BADARG;
-            if (!a->skip_score) {
-                rc = rope_qk_reverse(q, H, qsh, qsl, k, KVH, ksh, ksl, L, D, c, s, n_pos_tab, sec, a->inv_scale2, qu, ku,
-                                     (cudaStream_t)stream);
-                if (rc) return rc;
-            }
-        }
-        q = qu; k = ku; qsh = ksh = L * D; qsl = ksl = D;
-    }
-    if (!a->skip_score) {
-        ScoreBatch sb = {};
-        sb.n = 1; sb.H = H; sb.KVH = KVH; sb.L = L; sb.D = D;
-        sb.q[0] = q; sb.k[0] = k; sb.head_scores[0] = a->head_scores;
-        sb.q_stride_h[0] = qsh; sb.q_stride_l[0] = qsl; sb.k_stride_h[0] = ksh; sb.k_stride_l[0] = ksl;
-        if (a->keymask && key_elision_enabled()) {
-            // key patches keep score 1.0 whatever their column sum is: pass 2 only visits the other keys
-            if ((ksh | ksl) % 8 != 0 || D % 8 != 0 || ((uintptr_t)k & 15u) != 0) return RTK_E_ALIGN;
-            KeyElide ke = {};
-            ke.L = (int)L; ke.KVH = (int)KVH; ke.D = (int)D;
-            ke.keymask[0] = a->keymask; ke.slot[0] = slot_ws; ke.k[0] = (const __nv_bfloat16*)k;
-            ke.k_stride_h[0] = ksh; ke.k_stride_l[0] = ksl; ke.kc[0] = (__nv_bfloat16*)kc_ws; ke.n_keys = nkeys_ws;
-            rc = key_elide_prepare(ke, 1, sb, (cudaStream_t)stream);
-            if (rc) return rc;
-        }
-        if (a->ev_score_begin) cudaEventRecord((cudaEvent_t)a->ev_score_begin, (cudaStream_t)stream);
-        rc = pivot_score_batch(sb, score_ws, rtk_pivot_score_workspace_bytes(H, L), (cudaStream_t)stream);
-        if (rc) return rc;
-        if (a->ev_score_end) cudaEventRecord((cudaEvent_t)a->ev_score_end, (cudaStream_t)stream);
-    }
-    if (a->skip_select) {
-        if (xchg) {
-            // this rank's rows go into every peer's buffer, then the flags go up: one CTA, NVLink stores
-            XchgPut xp = {};
-            xp.src = (const __nv_bfloat16*)a->head_scores;
-            xp.n = (long long)KVH * L;
-            xp.world = a->xchg_world; xp.rank = a->xchg_rank; xp.epoch = a->xchg_epoch;
-            for (int r = 0; r < a->xchg_world; ++r) {
-                xp.dst[r] = (__nv_bfloat16*)a->xchg_scores[r] + (size_t)a->xchg_rank * KVH * L;
-                xp.flags[r] = a->xchg_flags[r];
-            }
-            RTK_LAUNCH_PDL(pivot_xchg_put_kernel, 1, 1024, 0, (cudaStream_t)stream, xp);
-        }
-        return 0;
-    }
-    {
-        if (a->keep < 1 || a->keep > L) return RTK_E_BADARG;
-        if (L > 16384) return RTK_E_UNSUPPORTED;
-        const size_t smem = (size_t)L * 4 + 112 * 4;
-        cudaError_t e = cudaFuncSetAttribute(pivot_select_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-        if (e != cudaSuccess) return (int)e;
-        RTK_LAUNCH_PDL(pivot_select_kernel, 1, kSelThreads, smem, (cudaStream_t)stream, (const __nv_bfloat16*)a->head_scores,
-                       (int)score_rows, (int)L, a->keymask, (int)a->keep, a->keep_idx, (__nv_bfloat16*)nullptr,
-                       (const long long*)(a->reforge ? a->pos : nullptr), a->reforge ? tmin : (long long*)nullptr,
-                       (const uint32_t*)(xchg ? a->xchg_flags[a->xchg_rank] : nullptr), xchg ? a->xchg_world : 0, a->xchg_epoch,
-                       xchg_timeout_ns());
-    }
-    // K (possibly the un-rotated copy), V (caller's strides), positions and - on the fast path - the forward rotation
-    // at the re-indexed positions: one launch, one CTA per kept token
-    {
-        if ((((uintptr_t)k | (uintptr_t)a->v | (uintptr_t)a->k_out | (uintptr_t)a->v_out) & 15u) != 0) return RTK_E_ALIGN;
-        if ((ksh | ksl | a->v_stride_h | a->v_stride_l | a->out_stride_h) % 8 != 0 || D % 16 != 0 || D > 256) return RTK_E_ALIGN;
-        if (a->pos && (!a->pos_out || a->n_pos < 1 || a->n_pos > 3)) return RTK_E_BADARG;
-        CompactParams p;
-        p.KVH = (int)KVH; p.L = (int)L; p.D = (int)D; p.keep = (int)a->keep; p.n_pos = a->pos ? a->n_pos : 0; p.reforge = a->reforge;
-        p.stride_h = ksh; p.stride_l = ksl; p.out_stride_h = a->out_stride_h;
-        p.v_stride_h = a->v_stride_h; p.v_stride_l = a->v_stride_l;
-        p.pos_out_stride = a->pos_out_stride > 0 ? a->pos_out_stride : a->keep;
-        p.ratio = (float)((double)a->keep / (double)L);
-        RopeParams rp = {};
-        rp.D = (int)D; rp.n_pos = a->n_pos; rp.L = (int)a->keep;
-        int acc = 0;
-        for (int i = 0; i < 6; ++i) {
-            acc += (a->n_pos == 3) ? a->mrope_section[i % 3] : 0;
-            rp.bound[i] = acc;
-        }
-        RTK_LAUNCH_PDL(pivot_compact_rope_kernel, (unsigned)a->keep, 128, 0, (cudaStream_t)stream, (const __nv_bfloat16*)k,
-                       (const __nv_bfloat16*)a->v, (const int32_t*)a->keep_idx, (__nv_bfloat16*)a->k_out, (__nv_bfloat16*)a->v_out,
-                       (const long long*)a->pos, (long long*)a->pos_out, (const long long*)tmin, a->inv_freq, a->attention_scaling, p,
-                       rp, fused_tables ? 1 : 0);
-    }
-    return 0;
-}
 
 extern "C" size_t rtk_pivot_update_batch_workspace_bytes(int64_t H, int64_t KVH, int64_t L, int64_t D, int64_t n_layers) {
     if (H < 1 || KVH < 1 || L < 1 || D < 1 || n_layers < 1) return 0;
@@ -1108,11 +877,16 @@ extern "C" size_t rtk_pivot_update_batch_workspace_bytes(int64_t H, int64_t KVH,
            n * key_elide_bytes(KVH, L, D) + 256;
 }
 
+extern "C" size_t rtk_pivot_update_workspace_bytes(int64_t H, int64_t KVH, int64_t L, int64_t D) {
+    return rtk_pivot_update_batch_workspace_bytes(H, KVH, L, D, 1);
+}
+
 #ifndef RTK_UNROT_TOKEN_MAJOR
-#define RTK_UNROT_TOKEN_MAJOR 1     // batched path: un-rotated copies laid out [L, heads, D] like the attention's own tensors
+#define RTK_UNROT_TOKEN_MAJOR 1     // un-rotated copies laid out [L, heads, D] like the attention's own tensors
 #endif
 
-// one group of <= kMaxBatchLayers layers
+// The update chain of one group of <= kMaxBatchLayers layers whose arguments update_check accepted: un-rotate, score,
+// exchange, select, compact + rotate.
 static int pivot_update_group(const rtk_pivot_update_args* a, int n, char* ws, cudaStream_t st) {
     const rtk_pivot_update_args& a0 = a[0];
     const int64_t H = a0.H, KVH = a0.KVH, L = a0.L, D = a0.D;
@@ -1162,19 +936,21 @@ static int pivot_update_group(const rtk_pivot_update_args* a, int n, char* ws, c
     rp.out_stride_h = uq_sh; rp.out_stride_l = uq_sl;
     rp.heads2 = (int)KVH; rp.out_stride_h2 = uk_sh; rp.out_stride_l2 = uk_sl;
     rp.inv_scale2 = a0.inv_scale2;
-    int acc = 0;
-    for (int i = 0; i < 6; ++i) {
-        acc += (a0.n_pos == 3) ? a0.mrope_section[i % 3] : 0;
-        rp.bound[i] = acc;
-    }
+    mrope_bounds(a0.n_pos, a0.mrope_section, D, rp.bound);
     const bool xchg = a0.xchg_world > 1;
     const int64_t score_rows = a0.score_rows > 0 ? a0.score_rows : KVH;
-    if (reforge) {
-        if (a0.n_pos == 3 && acc != D) return RTK_E_UNSUPPORTED;
-        // (skip_score: the un-rotated copies of the preceding skip_select call are still in the workspace)
-        if (!a0.skip_score)
+    // (skip_score: the un-rotated copies of the preceding skip_select call are still in the workspace)
+    if (reforge && !a0.skip_score) {
+        if (a0.inv_freq) {
             RTK_LAUNCH_PDL(pivot_unrope_qk_batch_kernel, dim3((unsigned)((L + kUnropeTok - 1) / kUnropeTok), (unsigned)n), 256, 0, st, t, a0.inv_freq,
                            a0.attention_scaling, rp);
+        } else {
+            // opaque rotary callable (one layer): un-rotate with the cos / sin tables it returned
+            rp.stride_h = a0.q_stride_h; rp.stride_l = a0.q_stride_l;
+            rp.x2 = t.k_in[0]; rp.out2 = t.ku[0]; rp.stride_h2 = a0.k_stride_h; rp.stride_l2 = a0.k_stride_l;
+            const int rc = rope_launch(a0.q, a0.cos, a0.sin, t.qu[0], rp, st);
+            if (rc) return rc;
+        }
     }
     if (!a0.skip_score) {
         bool any_mask = false;
@@ -1225,6 +1001,8 @@ static int pivot_update_group(const rtk_pivot_update_args* a, int n, char* ws, c
                        xchg ? a0.xchg_world : 0, a0.xchg_epoch, xchg_timeout_ns());
     }
     {
+        // K (the un-rotated copy when re-forging), V, positions and - with inv_freq - the forward rotation at the
+        // re-indexed positions; with cos / sin tables the caller rotates the kept keys itself (rtk_pivot_rope)
         CompactParams p = {};
         p.KVH = (int)KVH; p.L = (int)L; p.D = (int)D; p.keep = (int)a0.keep; p.n_pos = a0.pos ? a0.n_pos : 0; p.reforge = a0.reforge;
         p.ratio = (float)((double)a0.keep / (double)L);
@@ -1232,28 +1010,35 @@ static int pivot_update_group(const rtk_pivot_update_args* a, int n, char* ws, c
         rq.D = (int)D; rq.n_pos = a0.n_pos; rq.L = (int)a0.keep;
         for (int i = 0; i < 6; ++i) rq.bound[i] = rp.bound[i];
         RTK_LAUNCH_PDL(pivot_compact_rope_batch_kernel, dim3((unsigned)a0.keep, (unsigned)n), 128, 0, st, t, (const long long*)tmin,
-                       a0.inv_freq, a0.attention_scaling, p, rq, reforge ? 1 : 0);
+                       a0.inv_freq, a0.attention_scaling, p, rq, (reforge && a0.inv_freq) ? 1 : 0);
     }
     return 0;
 }
 
-extern "C" int rtk_pivot_update_batch(const rtk_pivot_update_args* layers, int64_t n_layers, void* workspace,
-                                      size_t workspace_bytes, void* stream) {
-    RTK_NVTX("rtk_pivot_update_batch");
-    if (!layers || n_layers < 1 || !workspace) return RTK_E_BADARG;
+// Every argument of an update of n layers (one chunk), checked before anything is launched.  A call that skips a step
+// is not checked for what only that step reads: the scoring reads q and k, the selection and compaction read keep, V,
+// the outputs and - when nothing is re-forged - k.
+static int update_check(const rtk_pivot_update_args* layers, int64_t n, const void* workspace, size_t workspace_bytes) {
+    if (!layers || n < 1 || !workspace) return RTK_E_BADARG;
     const rtk_pivot_update_args& a0 = layers[0];
-    if (a0.H < 1 || a0.KVH < 1 || a0.L < 1 || a0.keep < 1 || a0.keep > a0.L) return RTK_E_BADARG;
+    const bool scores = !a0.skip_score, selects = !a0.skip_select, xchg = a0.xchg_world > 1;
+    if (!scores && !selects) return RTK_E_BADARG;
+    if (a0.H < 1 || a0.KVH < 1 || a0.L < 1 || (selects && (a0.keep < 1 || a0.keep > a0.L))) return RTK_E_BADARG;
     if (a0.L > 16384 || a0.D % 16 != 0 || a0.D > 256) return RTK_E_UNSUPPORTED;
-    if (a0.skip_select && a0.skip_score) return RTK_E_BADARG;
-    if (a0.xchg_world > 1) {
+    if (scores && ((a0.D != 64 && a0.D != 128) || a0.H % a0.KVH != 0 || a0.H > 256)) return RTK_E_UNSUPPORTED;   // pivot_score_batch
+    if (xchg) {
         // one flag set per call: the exchange covers one group of layers
-        if (n_layers > kMaxBatchLayers) return RTK_E_UNSUPPORTED;
-        if (a0.xchg_world > 8 || a0.xchg_rank < 0 || a0.xchg_rank >= a0.xchg_world || !(a0.skip_select || a0.skip_score)) return RTK_E_BADARG;
+        if (n > kMaxBatchLayers) return RTK_E_UNSUPPORTED;
+        if (a0.xchg_world > 8 || a0.xchg_rank < 0 || a0.xchg_rank >= a0.xchg_world || (scores && selects)) return RTK_E_BADARG;
     }
-    if (a0.reforge && !a0.inv_freq) return RTK_E_UNSUPPORTED;        // opaque rotary callables go through rtk_pivot_update
+    // the cos / sin tables of an opaque rotary callable are those of one layer; a batch re-forges with inv_freq
+    if (a0.reforge && !a0.inv_freq && n > 1) return RTK_E_UNSUPPORTED;
+    // the mrope blocks are read by the un-rotation and, with inv_freq, by the compaction's forward rotation
+    int bound[6];
+    if (a0.reforge && (scores || a0.inv_freq) && !mrope_bounds(a0.n_pos, a0.mrope_section, a0.D, bound)) return RTK_E_UNSUPPORTED;
     if (((uintptr_t)workspace & 255u) != 0) return RTK_E_ALIGN;
-    if (workspace_bytes < rtk_pivot_update_batch_workspace_bytes(a0.H, a0.KVH, a0.L, a0.D, n_layers)) return RTK_E_WORKSPACE;
-    for (int64_t i = 0; i < n_layers; ++i) {
+    if (workspace_bytes < rtk_pivot_update_batch_workspace_bytes(a0.H, a0.KVH, a0.L, a0.D, n)) return RTK_E_WORKSPACE;
+    for (int64_t i = 0; i < n; ++i) {
         const rtk_pivot_update_args& x = layers[i];
         if (!x.q || !x.k || !x.v || !x.k_out || !x.v_out || !x.keep_idx || !x.head_scores) return RTK_E_BADARG;
         if (x.H != a0.H || x.KVH != a0.KVH || x.L != a0.L || x.D != a0.D || x.keep != a0.keep || x.reforge != a0.reforge ||
@@ -1264,23 +1049,51 @@ extern "C" int rtk_pivot_update_batch(const rtk_pivot_update_args* layers, int64
             return RTK_E_UNSUPPORTED;                                 // one chunk: the layers share shape and rotary
         for (int j = 0; j < 3; ++j)
             if (x.mrope_section[j] != a0.mrope_section[j]) return RTK_E_UNSUPPORTED;
-        if (x.reforge && (!x.pos || !x.pos_out)) return RTK_E_BADARG;
-        if (a0.xchg_world > 1)
+        if (x.reforge && (!x.pos || !x.pos_out || (!x.inv_freq && (!x.cos || !x.sin)))) return RTK_E_BADARG;
+        if (xchg) {
             for (int r = 0; r < a0.xchg_world; ++r)
                 if (!x.xchg_scores[r] || !a0.xchg_flags[r]) return RTK_E_BADARG;
-        if (a0.xchg_world > 1) {
+            // where the rows live is part of the protocol
             const char* own = (const char*)x.xchg_scores[a0.xchg_rank];
             if (a0.skip_score && (const char*)x.head_scores != own) return RTK_E_BADARG;
             if (a0.skip_select && (const char*)x.head_scores != own + (size_t)a0.xchg_rank * a0.KVH * a0.L * 2) return RTK_E_BADARG;
         }
-        if (x.pos && (!x.pos_out || x.n_pos < 1 || x.n_pos > 3)) return RTK_E_BADARG;
-        if ((((uintptr_t)x.q | (uintptr_t)x.k | (uintptr_t)x.v | (uintptr_t)x.k_out | (uintptr_t)x.v_out) & 15u) != 0) return RTK_E_ALIGN;
-        if ((x.q_stride_h | x.q_stride_l | x.k_stride_h | x.k_stride_l | x.v_stride_h | x.v_stride_l | x.out_stride_h) % 8 != 0)
-            return RTK_E_ALIGN;
+        if (x.pos && (selects || x.reforge) && (!x.pos_out || x.n_pos < 1 || x.n_pos > 3)) return RTK_E_BADARG;
+        uintptr_t ptrs = 0;
+        int64_t strides = 0;
+        if (scores) {
+            ptrs |= (uintptr_t)x.q;
+            strides |= x.q_stride_h | x.q_stride_l;
+        }
+        if (scores || !x.reforge) {
+            ptrs |= (uintptr_t)x.k;
+            strides |= x.k_stride_h | x.k_stride_l;
+        }
+        if (selects) {
+            ptrs |= (uintptr_t)x.v | (uintptr_t)x.k_out | (uintptr_t)x.v_out;
+            strides |= x.v_stride_h | x.v_stride_l | x.out_stride_h;
+        }
+        if ((ptrs & 15u) != 0 || strides % 8 != 0) return RTK_E_ALIGN;
     }
+    return 0;
+}
+
+extern "C" int rtk_pivot_update(const rtk_pivot_update_args* a, void* stream) {
+    RTK_NVTX("rtk_pivot_update");
+    if (!a) return RTK_E_BADARG;
+    const int rc = update_check(a, 1, a->workspace, a->workspace_bytes);
+    if (rc) return rc;
+    return pivot_update_group(a, 1, (char*)a->workspace, (cudaStream_t)stream);
+}
+
+extern "C" int rtk_pivot_update_batch(const rtk_pivot_update_args* layers, int64_t n_layers, void* workspace,
+                                      size_t workspace_bytes, void* stream) {
+    RTK_NVTX("rtk_pivot_update_batch");
+    int rc = update_check(layers, n_layers, workspace, workspace_bytes);
+    if (rc) return rc;
     for (int64_t i = 0; i < n_layers; i += kMaxBatchLayers) {
         const int n = (int)((n_layers - i) < kMaxBatchLayers ? (n_layers - i) : kMaxBatchLayers);
-        const int rc = pivot_update_group(layers + i, n, (char*)workspace, (cudaStream_t)stream);
+        rc = pivot_update_group(layers + i, n, (char*)workspace, (cudaStream_t)stream);
         if (rc) return rc;
     }
     return 0;
