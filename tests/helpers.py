@@ -12,6 +12,14 @@ def load_golden(name):
         return torch.load(io.BytesIO(f.read()))
 
 
+def bf16_round(x):
+    """round a float64 tensor to the nearest bf16 value (ties to even) in one step, kept as float64; below 2^-126 the
+    spacing stays 2^-133, as for bf16 subnormals"""
+    _, e = torch.frexp(x)
+    quantum = torch.ldexp(torch.ones_like(x), (e.clamp_min(-125) - 8).double())
+    return torch.round(x / quantum) * quantum
+
+
 class TableRotary:
     """Deterministic stand-in for the HF rotary module: callable (x, position_ids) -> (cos, sin)
     with ``attention_scaling`` (``longvideo_cache.py:249,256``).  YaRN-like scaling 1.1386."""

@@ -14,7 +14,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from helpers import scene_video
+from helpers import bf16_round, scene_video
 from test_gpu_fuzz import _ref_dpselect_indices
 from test_gpu_pivotkv import _cfg, _check_keep, _lc, qkv, ref_head_scores_cuda, ulp_diff
 
@@ -221,12 +221,6 @@ def test_mallm_sync_mode_at_the_limit(hard):
 
 
 # ============================================================================================================= PivotKV
-def _bf16_round(x):
-    """round a float64 tensor to the nearest bf16 value (ties to even) in one step, kept as float64"""
-    m, e = torch.frexp(x)
-    return torch.ldexp(torch.round(m * 256.0) / 256.0, e.double())
-
-
 def test_head_scores_fp64_anchor_at_the_length_limit():
     """Two query heads on one KV head at L = 16384 against the reference's chain with exact dot products: fp64 Q.K^T (exact
     for bf16 inputs with D = 128 terms), rounded to bf16 where the reference rounds (QK^T, / sqrt(D), softmax, sum, mean),
@@ -240,12 +234,12 @@ def test_head_scores_fp64_anchor_at_the_length_limit():
     kd = k[0, 0].double()
     s = torch.empty(H, L, dtype=torch.float64, device="cuda")
     for h in range(H):                                                               # one [L, L] fp64 plane at a time
-        w = _bf16_round(torch.matmul(q[0, h].double(), kd.t()))
+        w = bf16_round(torch.matmul(q[0, h].double(), kd.t()))
         w = (w.to(BF) / math.sqrt(D)).double()                                       # the reference's bf16 / python float
-        w = _bf16_round(torch.softmax(w, dim=-1))
-        s[h] = _bf16_round(w.sum(0))                                                 # sum over the queries
+        w = bf16_round(torch.softmax(w, dim=-1))
+        s[h] = bf16_round(w.sum(0))                                                 # sum over the queries
         del w
-    anchor = _bf16_round(s.reshape(KVH, H // KVH, L).mean(1)).to(BF)
+    anchor = bf16_round(s.reshape(KVH, H // KVH, L).mean(1)).to(BF)
     d_kernel = ulp_diff(got, anchor)
     d_cublas = ulp_diff(cublas, anchor)
     print(f"\nfp64 anchor, L={L}: kernel max {int(d_kernel.max())} ulp on {float((d_kernel > 0).float().mean()):.4%}, "
