@@ -146,14 +146,16 @@ def test_dpselect_distance_at_the_patch_limit():
 
 
 # ============================================================================================================== MA-LLM
-# rtk_mallm_compress, sync = 0: the per-patch state stays in shared memory while 25*T + 4*C + 32 bytes (+ 1 KB for the
-# kernel's static shared memory) fit; beyond that mallm_rounds_kernel keeps it in global memory
+# rtk_mallm_compress, sync = 0: the per-patch state (25 bytes per frame) stays in shared memory together with two row
+# buffers while 25*T + 4*C + 32 bytes (+ 1 KB for the kernel's static shared memory) fit, and with one row buffer
+# beyond that.  `where` names the side of that switch: "smem" = two buffers, "global" and "limit" = one buffer.
 def _mallm_smem_fits(T, C):
+    """two row buffers fit"""
     return 25 * T + 4 * C + 32 + 1024 <= _optin()
 
 
 def _mallm_tg(C):
-    """first T whose per-patch state no longer fits into shared memory (7945 at C = 8192 on a B200)"""
+    """first T at which two row buffers no longer fit (7945 at C = 8192 on a B200)"""
     return (_optin() - 4 * C - 32 - 1024) // 25 + 1
 
 
@@ -199,12 +201,13 @@ def test_mallm_patch_mode_around_the_shared_memory_switch(where, N, hard, dt):
     C = 8192
     T = _mallm_T(where, C)
     assert T <= 8192 and _mallm_smem_fits(T, C) == (where == "smem")
+    assert 25 * 8192 + 2 * 8192 + 32 + 1024 <= _optin()        # one buffer fits up to the limit: the host never refuses
     _mallm_check(_mallm_bank(T, N, C), T - dt, False, hard)
 
 
 @pytest.mark.parametrize("hard", [False, True])
 def test_mallm_patch_mode_thousands_of_rounds(hard):
-    """N = 1, t = T/2 on the global-memory path: about 4000 merges of one patch column"""
+    """N = 1, t = T/2 with one row buffer: about 4000 merges of one patch column"""
     C = 8192
     T = _mallm_tg(C)
     assert not _mallm_smem_fits(T, C)

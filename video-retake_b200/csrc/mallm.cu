@@ -10,8 +10,10 @@
 //     of frames m and next(m), and the replay of the reference's `x = rd(rd(x * size) / size)` on the rows for
 //     which that map is not yet at a fixed point (it is idempotent after one or two applications, so the "dirty"
 //     list holds the rows changed in the previous round only), then the similarities next to changed rows;
-//   * patch-local mode runs all rounds of a patch column inside one CTA of one launch; sync mode shares one argmax
-//     over the bf16 mean of the similarities across patches (one round kernel + one argmax kernel per round).
+//   * one round body (mallm_round) serves both modes, over a patch column whose state lives in shared memory or in
+//     the workspace: patch-local mode runs all rounds of a patch column inside one CTA of one launch, the state in
+//     shared memory; sync mode shares one argmax over the bf16 mean of the similarities across patches (one argmax
+//     kernel + one round kernel per round, the state in the workspace).
 //
 // Arithmetic is the reference's, bit for bit (bf16 bank): rd() = round to nearest even to bf16 after EVERY op,
 // true fp32 division, sizes kept in bf16; cosine similarity as in dpselect.cu (ATen reduction orders: 4-element
@@ -49,11 +51,6 @@ struct MallmParams {
 };
 
 __device__ __forceinline__ size_t at(const MallmParams& P, int i, int p) { return (size_t)i * P.si + (size_t)p * P.sp; }
-
-__device__ __forceinline__ const __nv_bfloat16* row_ptr(const MallmParams& P, int i, int p) {
-    const size_t off = ((size_t)i * P.N + p) * (size_t)P.C;
-    return (!P.hard && P.in_work[at(P, i, p)]) ? P.work + off : P.x + off;
-}
 
 // clamp_min_(bf16(1e-8)) of F.cosine_similarity
 __device__ __forceinline__ float clamp_norm(float ss) {
@@ -201,351 +198,272 @@ __device__ __forceinline__ uint32_t rescale_pair(uint32_t a, float s) {
     return pack_bf16x2_rn(lo, hi);
 }
 
-// soft merge of frames m and next(m) of patch p by the whole CTA; `round` = number of merges already done;
-// simv[i * sstride] is the patch's similarity column (global state, or the shared-memory copy of the persistent loop)
-__device__ __forceinline__ void mallm_soft_round(const MallmParams& P, int p, int round, int m, float* simv, long long sstride) {
-    __shared__ int s_n, s_cnt;
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int T = P.T, C = P.C;
-    if (threadIdx.x == 0) {
-        s_n = P.next[at(P, m, p)];
-        s_cnt = 0;
+// Row i of patch p: the input row, or its copy in the workspace once a merge or replay has rewritten it.
+__device__ __forceinline__ const __nv_bfloat16* bank_row(const MallmParams& P, int i, int p, bool in_work) {
+    const size_t off = ((size_t)i * P.N + p) * (size_t)P.C;
+    return in_work ? P.work + off : P.x + off;
+}
+__device__ __forceinline__ __nv_bfloat16* work_row(const MallmParams& P, int i, int p) {
+    return P.work + ((size_t)i * P.N + p) * (size_t)P.C;
+}
+
+// The state of one patch column, as the round body sees it.  Two implementations: GlobalColumn reads and writes the
+// workspace arrays (sync mode, where every round is its own launch), SmemColumn keeps the column in shared memory for
+// all rounds of one launch (patch-local mode) and mirrors to the workspace only what mallm_emit_kernel reads.
+struct GlobalColumn {
+    const MallmParams& P;
+    const int p;
+    __device__ GlobalColumn(const MallmParams& P_, int p_) : P(P_), p(p_) {}
+    __device__ float& sim(int i) const { return P.sim[at(P, i, p)]; }
+    __device__ float& nrm(int i) const { return P.nrm[at(P, i, p)]; }
+    __device__ int& next(int i) const { return P.next[at(P, i, p)]; }
+    __device__ int& prev(int i) const { return P.prev[at(P, i, p)]; }
+    __device__ float size(int i) const { return P.size[at(P, i, p)]; }
+    __device__ void set_size(int i, float s) const { P.size[at(P, i, p)] = s; }
+    __device__ const __nv_bfloat16* row(int i) const { return bank_row(P, i, p, !P.hard && P.in_work[at(P, i, p)]); }
+    __device__ void set_in_work(int i) const { P.in_work[at(P, i, p)] = 1; }
+    // the rows whose similarity changed in round r: mallm_sync_argmax_kernel refreshes their mean
+    __device__ void stamp(int i, int r) const { P.touched[i] = r + 1; }
+    __device__ void kill(int i, int r) const {
+        P.alive[at(P, i, p)] = 0;
+        sim(i) = -INFINITY;
+        stamp(i, r);
     }
-    __syncthreads();
-    const int n = s_n;
-    const int* cur = P.dirty + ((size_t)(round & 1) * P.N + p) * T;
-    int* nxt = P.dirty + ((size_t)((round + 1) & 1) * P.N + p) * T;
-    const int nd = P.n_dirty[(size_t)(round & 1) * P.N + p];
-    const size_t row_elems = (size_t)C;
-    // ---- row tasks: task 0 merges (m, n) into m; task k > 0 replays x = rd(rd(x * s) / s) on a dirty row
-    for (int task = warp; task <= nd; task += kMlWarps) {
-        const int j = task ? cur[task - 1] : m;
-        if (task && (j == m || j == n)) continue;
-        const size_t a = at(P, j, p);
-        const uint2* src = reinterpret_cast<const uint2*>(row_ptr(P, j, p));
-        uint2* dst = reinterpret_cast<uint2*>(P.work + ((size_t)j * P.N + p) * row_elems);
-        float a0 = 0.f, a1 = 0.f, a2 = 0.f, a3 = 0.f;
-        bool changed = true;
-        const int nv = C >> 2;
-        if (task == 0) {
-            const uint2* src2 = reinterpret_cast<const uint2*>(row_ptr(P, n, p));
-            const float sa = P.size[a], sb = P.size[at(P, n, p)];
-            const float snew = round_bf16(sa + sb);
-            auto step = [&](int v, const uint2& q, const uint2& r) {
-                uint2 y;
-                y.x = merge_pair(q.x, r.x, sa, sb, snew);
-                y.y = merge_pair(q.y, r.y, sa, sb, snew);
-                dst[v] = y;
-                fma_sq_bf16x2(a0, a1, y.x);
-                fma_sq_bf16x2(a2, a3, y.y);
-            };
-            constexpr int kHalf = kBatch / 2;
-            int v = lane;
-            for (; v + (kHalf - 1) * 32 < nv; v += kHalf * 32) {
-                uint2 q[kHalf], r[kHalf];
-#pragma unroll
-                for (int u = 0; u < kHalf; ++u) { q[u] = src[v + 32 * u]; r[u] = src2[v + 32 * u]; }
-#pragma unroll
-                for (int u = 0; u < kHalf; ++u) step(v + 32 * u, q[u], r[u]);
-            }
-            for (; v < nv; v += 32) step(v, src[v], src2[v]);
-            if (lane == 0) P.size[a] = snew;
-        } else {
-            const float s = P.size[a];
-            bool diff = false;
-            auto step = [&](int v, const uint2& q) {
-                uint2 y;
-                y.x = rescale_pair(q.x, s);
-                y.y = rescale_pair(q.y, s);
-                diff |= (y.x != q.x) || (y.y != q.y);
-                dst[v] = y;
-                fma_sq_bf16x2(a0, a1, y.x);
-                fma_sq_bf16x2(a2, a3, y.y);
-            };
-            int v = lane;
-            for (; v + (kBatch - 1) * 32 < nv; v += kBatch * 32) {
-                uint2 q[kBatch];
-#pragma unroll
-                for (int u = 0; u < kBatch; ++u) q[u] = src[v + 32 * u];
-#pragma unroll
-                for (int u = 0; u < kBatch; ++u) step(v + 32 * u, q[u]);
-            }
-            for (; v < nv; v += 32) step(v, src[v]);
-            changed = __any_sync(0xffffffffu, diff);
-        }
-        const float nr = clamp_norm(warp_tree(((a0 + a1) + a2) + a3, lane));
-        if (lane == 0) {
-            P.nrm[a] = nr;
-            P.in_work[a] = 1;
-            if (changed) nxt[atomicAdd(&s_cnt, 1)] = j;
-        }
+    // dirty lists [2][N][T] with their counts [2][N]: list r & 1 is read in round r, list (r + 1) & 1 written
+    __device__ int n_dirty(int r) const { return P.n_dirty[(size_t)(r & 1) * P.N + p]; }
+    __device__ int dirty(int r, int k) const { return P.dirty[((size_t)(r & 1) * P.N + p) * P.T + k]; }
+    __device__ void set_dirty(int r, int k, int i) const { P.dirty[((size_t)(r & 1) * P.N + p) * P.T + k] = i; }
+    __device__ void end_round(int r, int nch) const {
+        if (threadIdx.x == 0) P.n_dirty[(size_t)((r + 1) & 1) * P.N + p] = nch;
     }
-    __syncthreads();
-    if (threadIdx.x == 0) {                                      // unlink n
-        const int nx = P.next[at(P, n, p)];
-        P.next[at(P, m, p)] = nx;
-        if (nx < T) P.prev[at(P, nx, p)] = m;
-        P.alive[at(P, n, p)] = 0;
-        simv[(size_t)n * sstride] = -INFINITY;
-        if (P.sync && p == 0) P.touched[n] = round + 1;
-        P.n_dirty[(size_t)((round + 1) & 1) * P.N + p] = s_cnt;
+};
+
+struct SmemColumn {
+    const MallmParams& P;
+    const int p;
+    float *sim_, *nrm_, *size_;
+    int *next_, *prev_;
+    short* dirty_;               // [2][T]
+    uint8_t* in_work_;
+    int nd;                      // length of the dirty list the next round reads
+    __device__ float& sim(int i) const { return sim_[i]; }
+    __device__ float& nrm(int i) const { return nrm_[i]; }
+    __device__ int& next(int i) const { return next_[i]; }
+    __device__ int& prev(int i) const { return prev_[i]; }
+    __device__ float size(int i) const { return size_[i]; }
+    __device__ void set_size(int i, float s) const {
+        size_[i] = s;
+        P.size[at(P, i, p)] = s;
+    }
+    __device__ const __nv_bfloat16* row(int i) const { return bank_row(P, i, p, !P.hard && in_work_[i]); }
+    __device__ void set_in_work(int i) const {
+        in_work_[i] = 1;
+        P.in_work[at(P, i, p)] = 1;
+    }
+    __device__ void stamp(int, int) const {}
+    __device__ void kill(int i, int) const {
+        P.alive[at(P, i, p)] = 0;
+        sim_[i] = -INFINITY;
+    }
+    __device__ int n_dirty(int) const { return nd; }
+    __device__ int dirty(int r, int k) const { return dirty_[(size_t)(r & 1) * P.T + k]; }
+    __device__ void set_dirty(int r, int k, int i) const { dirty_[(size_t)(r & 1) * P.T + k] = (short)i; }
+    __device__ void end_round(int, int nch) { nd = nch; }
+};
+
+// Shared memory of patch-local mode: the column state (25 bytes per frame), then kBufs row buffers.  The host sizes the
+// launch with `bytes`, the kernel carves its arrays at the offsets.
+struct RoundsSmem {
+    size_t sim, nrm, size, next, prev, dirty, in_work, rowbuf, bytes;
+};
+__host__ __device__ inline RoundsSmem rounds_smem(int T, int C, int bufs) {
+    const size_t t4 = (size_t)T * 4;
+    RoundsSmem L;
+    L.sim = 0;
+    L.nrm = t4;
+    L.size = 2 * t4;
+    L.next = 3 * t4;
+    L.prev = 4 * t4;
+    L.dirty = 5 * t4;
+    L.in_work = 6 * t4;
+    L.rowbuf = ((size_t)T * 25 + 15) & ~(size_t)15;
+    L.bytes = (size_t)T * 25 + 16 + (size_t)bufs * C * 2 + 16;
+    return L;
+}
+
+// One round on one patch column, by the whole CTA; m is the frame the round merges (soft) or drops (hard).
+// Soft: the merge of (m, next(m)) into m and the replay of x = rd(rd(x * s) / s) on the dirty rows are element-wise over
+// the whole CTA, kBufs rows per batch with every load of the batch in flight at once; each result goes to the workspace
+// row AND to a shared row buffer (`rowbuf`, kBufs * C bf16) from which one warp per row takes the norm in ATen's order.
+// Then the similarities on both sides of every changed row, one warp per pair.  Hard: one pair similarity.
+template <int kBufs, class Col>
+__device__ __forceinline__ void mallm_round(const MallmParams& P, Col& c, __nv_bfloat16* rowbuf, int r, int m) {
+    __shared__ int s_cnt, s_changed[kBufs];
+    const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
+    const int T = P.T, C = P.C, nv = C >> 2;
+    if (P.hard) {
+        if (warp == 0) {
+            const int pm = c.prev(m), n = c.next(m);
+            float sv = 0.f;
+            if (pm >= 0) sv = warp_pair_sim(c.row(pm), c.nrm(pm), c.row(n), c.nrm(n), C, lane);
+            if (lane == 0) {
+                c.kill(m, r);
+                c.prev(n) = pm;
+                if (pm >= 0) {
+                    c.next(pm) = n;
+                    c.sim(pm) = sv;
+                    c.stamp(pm, r);
+                }
+            }
+        }
+        __syncthreads();
+        return;
+    }
+    const int n = c.next(m), nd = c.n_dirty(r);
+    if (tid == 0) s_cnt = 0;
+    // ---- row tasks in batches of kBufs: task 0 = merge (m, n) -> m, task k > 0 = replay on dirty row k - 1
+    for (int t0 = 0; t0 <= nd; t0 += kBufs) {
+        if (tid < kBufs) s_changed[tid] = 0;
+        __syncthreads();
+#pragma unroll
+        for (int k = 0; k < kBufs; ++k) {
+            const int task = t0 + k;
+            if (task > nd) break;
+            const int j = task ? c.dirty(r, task - 1) : m;
+            if (task && (j == m || j == n)) continue;
+            const uint2* src = reinterpret_cast<const uint2*>(c.row(j));
+            uint2* dst = reinterpret_cast<uint2*>(work_row(P, j, c.p));
+            uint2* buf = reinterpret_cast<uint2*>(rowbuf + (size_t)k * C);
+            if (task == 0) {
+                const uint2* src2 = reinterpret_cast<const uint2*>(c.row(n));
+                const float sa = c.size(m), sb = c.size(n);
+                const float snew = round_bf16(sa + sb);
+                for (int v0 = tid; v0 < nv; v0 += 4 * kMlThreads) {
+                    uint2 q[4], w[4];
+#pragma unroll
+                    for (int u = 0; u < 4; ++u) {
+                        const int v = v0 + u * kMlThreads;
+                        if (v < nv) { q[u] = src[v]; w[u] = src2[v]; }
+                    }
+#pragma unroll
+                    for (int u = 0; u < 4; ++u) {
+                        const int v = v0 + u * kMlThreads;
+                        if (v < nv) {
+                            uint2 y;
+                            y.x = merge_pair(q[u].x, w[u].x, sa, sb, snew);
+                            y.y = merge_pair(q[u].y, w[u].y, sa, sb, snew);
+                            dst[v] = y;
+                            buf[v] = y;
+                        }
+                    }
+                }
+                if (tid == 0) s_changed[k] = 1;
+            } else {
+                const float sz = c.size(j);
+                bool diff = false;
+                for (int v0 = tid; v0 < nv; v0 += 4 * kMlThreads) {
+                    uint2 q[4];
+#pragma unroll
+                    for (int u = 0; u < 4; ++u) {
+                        const int v = v0 + u * kMlThreads;
+                        if (v < nv) q[u] = src[v];
+                    }
+#pragma unroll
+                    for (int u = 0; u < 4; ++u) {
+                        const int v = v0 + u * kMlThreads;
+                        if (v < nv) {
+                            uint2 y;
+                            y.x = rescale_pair(q[u].x, sz);
+                            y.y = rescale_pair(q[u].y, sz);
+                            diff |= (y.x != q[u].x) || (y.y != q[u].y);
+                            dst[v] = y;
+                            buf[v] = y;
+                        }
+                    }
+                }
+                if (diff) s_changed[k] = 1;
+            }
+        }
+        __syncthreads();
+        if (warp < kBufs && t0 + warp <= nd) {
+            const int task = t0 + warp;
+            const int j = task ? c.dirty(r, task - 1) : m;
+            if (!(task && (j == m || j == n))) {
+                const float nr = warp_row_norm(rowbuf + (size_t)warp * C, C, lane);
+                if (lane == 0) {
+                    c.nrm(j) = nr;
+                    c.set_in_work(j);
+                    if (s_changed[warp]) c.set_dirty(r + 1, atomicAdd(&s_cnt, 1), j);
+                }
+            }
+        }
+        __syncthreads();
+    }
+    if (tid == 0) {                                              // sizes and links: n leaves the list
+        c.set_size(m, round_bf16(c.size(m) + c.size(n)));
+        const int nx = c.next(n);
+        c.next(m) = nx;
+        if (nx < T) c.prev(nx) = m;
+        c.kill(n, r);
     }
     __syncthreads();
     // ---- similarities on both sides of every changed row
     const int nch = s_cnt;
     for (int task = warp; task < 2 * nch; task += kMlWarps) {
-        const int j = nxt[task >> 1];
+        const int j = c.dirty(r + 1, task >> 1);
         int a, b;
-        if (task & 1) { a = j; b = P.next[at(P, j, p)]; }
-        else { a = P.prev[at(P, j, p)]; b = j; }
+        if (task & 1) { a = j; b = c.next(j); }
+        else { a = c.prev(j); b = j; }
         if (a < 0) continue;
-        float s = -INFINITY;
-        if (b < T) s = warp_pair_sim(row_ptr(P, a, p), P.nrm[at(P, a, p)], row_ptr(P, b, p), P.nrm[at(P, b, p)], C, lane);
+        float sv = -INFINITY;
+        if (b < T) sv = warp_pair_sim(c.row(a), c.nrm(a), c.row(b), c.nrm(b), C, lane);
         if (lane == 0) {
-            simv[(size_t)a * sstride] = s;
-            if (P.sync) P.touched[a] = round + 1;
+            c.sim(a) = sv;
+            c.stamp(a, r);
         }
     }
+    c.end_round(r, nch);
+    __syncthreads();
 }
 
-// hard variant: frame m is deleted, nothing is rewritten (one warp's work)
-__device__ __forceinline__ void mallm_hard_round(const MallmParams& P, int p, int round, int m, float* simv, long long sstride) {
-    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    if (warp != 0) return;
-    const int pm = P.prev[at(P, m, p)], n = P.next[at(P, m, p)];
-    float s = 0.f;
-    if (pm >= 0) s = warp_pair_sim(row_ptr(P, pm, p), P.nrm[at(P, pm, p)], row_ptr(P, n, p), P.nrm[at(P, n, p)], P.C, lane);
-    if (lane == 0) {
-        P.alive[at(P, m, p)] = 0;
-        simv[(size_t)m * sstride] = -INFINITY;
-        P.prev[at(P, n, p)] = pm;
-        if (pm >= 0) {
-            P.next[at(P, pm, p)] = n;
-            simv[(size_t)pm * sstride] = s;
-        }
-        if (P.sync && p == 0) {
-            P.touched[m] = round + 1;
-            if (pm >= 0) P.touched[pm] = round + 1;
-        }
-    }
-}
-
-// one round per launch (sync mode: the shared argmax comes from mallm_sync_argmax_kernel of the previous launch)
+// sync mode, one round per launch: every patch merges or drops the frame of the shared argmax (merge_at[0], from
+// mallm_sync_argmax_kernel); dynamic shared memory = the row buffers, kSyncBufs * C * 2 bytes (at most 32 KB)
+constexpr int kSyncBufs = 2;
 __global__ void __launch_bounds__(kMlThreads) mallm_round_kernel(MallmParams P, int round) {
     pdl_enter();
-    __shared__ Best s_best[kMlWarps];
-    const int p = blockIdx.x;
-    float* simv = P.sim + (size_t)p * P.sp;
-    const int m = P.sync ? P.merge_at[0] : block_argmax(simv, P.si, P.T, s_best);
-    if (P.hard) mallm_hard_round(P, p, round, m, simv, P.si);
-    else mallm_soft_round(P, p, round, m, simv, P.si);
+    extern __shared__ __align__(16) uint8_t smem_raw[];
+    GlobalColumn c(P, blockIdx.x);
+    mallm_round<kSyncBufs>(P, c, reinterpret_cast<__nv_bfloat16*>(smem_raw), round, P.merge_at[0]);
 }
 
-// patch-local mode: ALL rounds of one patch column in one CTA, the similarity column lives in shared memory
+// patch-local mode: ALL rounds of one patch column in one CTA, the column state in shared memory (rounds_smem)
+template <int kBufs>
 __global__ void __launch_bounds__(kMlThreads) mallm_rounds_kernel(MallmParams P, int rounds) {
     pdl_enter();
     extern __shared__ __align__(16) uint8_t smem_raw[];
-    float* sim_s = reinterpret_cast<float*>(smem_raw);           // [T]
     __shared__ Best s_best[kMlWarps];
-    const int p = blockIdx.x;
-    for (int i = threadIdx.x; i < P.T; i += blockDim.x) sim_s[i] = P.sim[at(P, i, p)];
-    __syncthreads();
-    for (int r = 0; r < rounds; ++r) {
-        const int m = block_argmax(sim_s, 1, P.T, s_best);
-        if (P.hard) mallm_hard_round(P, p, r, m, sim_s, 1);
-        else mallm_soft_round(P, p, r, m, sim_s, 1);
-        __syncthreads();
-    }
-}
-
-
-// Patch-local mode, fast variant: the whole per-patch state (similarities, norms, sizes, links, flags, dirty lists)
-// lives in shared memory for all rounds, and the row work of a round is done by the whole CTA: the merge (and the
-// replay on dirty rows) is element-wise over 256 threads with every load of the round in flight at once, the result
-// goes to the workspace row AND to a shared-memory row buffer from which ONE warp then takes the norm in ATen's order.
-// Only `alive`, `in_work`, `size` (read by the emit kernel) and the rewritten rows go back to global memory.
-constexpr int kRowBufs = 2;      // row tasks handled per batch (merge + one dirty row is the common case)
-
-struct RoundsSmem {
-    float *sim, *nrm, *size;
-    int *next, *prev;
-    short* dirty;                // [2][T]
-    uint8_t* in_work;
-    __nv_bfloat16* rowbuf;       // [kRowBufs][C]
-};
-__host__ __device__ inline size_t rounds_smem_bytes(int T, int C) {
-    return (size_t)T * (5 * 4 + 2 * 2 + 1) + 16 + (size_t)kRowBufs * C * 2 + 16;
-}
-
-__global__ void __launch_bounds__(kMlThreads) mallm_rounds_smem_kernel(MallmParams P, int rounds) {
-    pdl_enter();
-    extern __shared__ __align__(16) uint8_t smem_raw[];
-    __shared__ Best s_best[kMlWarps];
-    __shared__ int s_cnt, s_changed[kRowBufs];
-    const int p = blockIdx.x, tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const int T = P.T, C = P.C, nv = C >> 2;
-    RoundsSmem S;
-    {
-        uint8_t* q = smem_raw;
-        S.sim = reinterpret_cast<float*>(q);   q += (size_t)T * 4;
-        S.nrm = reinterpret_cast<float*>(q);   q += (size_t)T * 4;
-        S.size = reinterpret_cast<float*>(q);  q += (size_t)T * 4;
-        S.next = reinterpret_cast<int*>(q);    q += (size_t)T * 4;
-        S.prev = reinterpret_cast<int*>(q);    q += (size_t)T * 4;
-        S.dirty = reinterpret_cast<short*>(q); q += (size_t)T * 4;
-        S.in_work = q;                         q += ((size_t)T + 15) & ~(size_t)15;
-        S.rowbuf = reinterpret_cast<__nv_bfloat16*>(q);
-    }
-    for (int i = tid; i < T; i += blockDim.x) {
+    const int p = blockIdx.x, T = P.T;
+    const RoundsSmem L = rounds_smem(T, P.C, kBufs);
+    SmemColumn c{P, p,
+                 reinterpret_cast<float*>(smem_raw + L.sim), reinterpret_cast<float*>(smem_raw + L.nrm),
+                 reinterpret_cast<float*>(smem_raw + L.size), reinterpret_cast<int*>(smem_raw + L.next),
+                 reinterpret_cast<int*>(smem_raw + L.prev), reinterpret_cast<short*>(smem_raw + L.dirty),
+                 smem_raw + L.in_work, P.hard ? 0 : P.n_dirty[p]};
+    for (int i = threadIdx.x; i < T; i += blockDim.x) {
         const size_t a = at(P, i, p);
-        S.sim[i] = P.sim[a];
-        S.nrm[i] = P.nrm[a];
-        S.next[i] = P.next[a];
-        S.prev[i] = P.prev[a];
+        c.sim_[i] = P.sim[a];
+        c.nrm_[i] = P.nrm[a];
+        c.next_[i] = P.next[a];
+        c.prev_[i] = P.prev[a];
         if (!P.hard) {
-            S.size[i] = P.size[a];
-            S.in_work[i] = P.in_work[a];
+            c.size_[i] = P.size[a];
+            c.in_work_[i] = P.in_work[a];
         }
     }
-    int nd = 0;
-    if (!P.hard) {
-        nd = P.n_dirty[p];
-        for (int i = tid; i < nd; i += blockDim.x) S.dirty[i] = (short)P.dirty[(size_t)p * T + i];
-    }
+    for (int k = threadIdx.x; k < c.nd; k += blockDim.x) c.set_dirty(0, k, P.dirty[(size_t)p * T + k]);
     __syncthreads();
-    auto row = [&](int i) -> const __nv_bfloat16* {
-        const size_t off = ((size_t)i * P.N + p) * (size_t)C;
-        return (!P.hard && S.in_work[i]) ? P.work + off : P.x + off;
-    };
-    for (int r = 0; r < rounds; ++r) {
-        const int m = block_argmax(S.sim, 1, T, s_best);
-        if (P.hard) {
-            if (warp == 0) {
-                const int pm = S.prev[m], n = S.next[m];
-                float sv = 0.f;
-                if (pm >= 0) sv = warp_pair_sim(row(pm), S.nrm[pm], row(n), S.nrm[n], C, lane);
-                if (lane == 0) {
-                    P.alive[at(P, m, p)] = 0;
-                    S.sim[m] = -INFINITY;
-                    S.prev[n] = pm;
-                    if (pm >= 0) {
-                        S.next[pm] = n;
-                        S.sim[pm] = sv;
-                    }
-                }
-            }
-            __syncthreads();
-            continue;
-        }
-        const int n = S.next[m];
-        const short* cur = S.dirty + (size_t)(r & 1) * T;
-        short* nxt = S.dirty + (size_t)((r + 1) & 1) * T;
-        if (tid == 0) s_cnt = 0;
-        // ---- row tasks in batches of kRowBufs: task 0 = merge (m, n) -> m, task k > 0 = replay on dirty row cur[k - 1]
-        for (int t0 = 0; t0 <= nd; t0 += kRowBufs) {
-            if (tid < kRowBufs) s_changed[tid] = 0;
-            __syncthreads();
-#pragma unroll
-            for (int k = 0; k < kRowBufs; ++k) {
-                const int task = t0 + k;
-                if (task > nd) break;
-                const int j = task ? cur[task - 1] : m;
-                if (task && (j == m || j == n)) continue;
-                const uint2* src = reinterpret_cast<const uint2*>(row(j));
-                uint2* dst = reinterpret_cast<uint2*>(P.work + ((size_t)j * P.N + p) * (size_t)C);
-                uint2* buf = reinterpret_cast<uint2*>(S.rowbuf + (size_t)k * C);
-                if (task == 0) {
-                    const uint2* src2 = reinterpret_cast<const uint2*>(row(n));
-                    const float sa = S.size[m], sb = S.size[n];
-                    const float snew = round_bf16(sa + sb);
-                    for (int v0 = tid; v0 < nv; v0 += 4 * kMlThreads) {
-                        uint2 q[4], w[4];
-#pragma unroll
-                        for (int u = 0; u < 4; ++u) {
-                            const int v = v0 + u * kMlThreads;
-                            if (v < nv) { q[u] = src[v]; w[u] = src2[v]; }
-                        }
-#pragma unroll
-                        for (int u = 0; u < 4; ++u) {
-                            const int v = v0 + u * kMlThreads;
-                            if (v < nv) {
-                                uint2 y;
-                                y.x = merge_pair(q[u].x, w[u].x, sa, sb, snew);
-                                y.y = merge_pair(q[u].y, w[u].y, sa, sb, snew);
-                                dst[v] = y;
-                                buf[v] = y;
-                            }
-                        }
-                    }
-                    if (tid == 0) s_changed[k] = 1;
-                } else {
-                    const float sz = S.size[j];
-                    bool diff = false;
-                    for (int v0 = tid; v0 < nv; v0 += 4 * kMlThreads) {
-                        uint2 q[4];
-#pragma unroll
-                        for (int u = 0; u < 4; ++u) {
-                            const int v = v0 + u * kMlThreads;
-                            if (v < nv) q[u] = src[v];
-                        }
-#pragma unroll
-                        for (int u = 0; u < 4; ++u) {
-                            const int v = v0 + u * kMlThreads;
-                            if (v < nv) {
-                                uint2 y;
-                                y.x = rescale_pair(q[u].x, sz);
-                                y.y = rescale_pair(q[u].y, sz);
-                                diff |= (y.x != q[u].x) || (y.y != q[u].y);
-                                dst[v] = y;
-                                buf[v] = y;
-                            }
-                        }
-                    }
-                    if (diff) s_changed[k] = 1;
-                }
-            }
-            __syncthreads();
-            if (warp < kRowBufs && t0 + warp <= nd) {
-                const int task = t0 + warp;
-                const int j = task ? cur[task - 1] : m;
-                if (!(task && (j == m || j == n))) {
-                    const float nr = warp_row_norm(S.rowbuf + (size_t)warp * C, C, lane);
-                    if (lane == 0) {
-                        S.nrm[j] = nr;
-                        S.in_work[j] = 1;
-                        P.in_work[at(P, j, p)] = 1;
-                        if (s_changed[warp]) nxt[atomicAdd(&s_cnt, 1)] = (short)j;
-                    }
-                }
-            }
-            __syncthreads();
-        }
-        if (tid == 0) {                                          // sizes and links
-            const float snew = round_bf16(S.size[m] + S.size[n]);
-            S.size[m] = snew;
-            P.size[at(P, m, p)] = snew;
-            const int nx = S.next[n];
-            S.next[m] = nx;
-            if (nx < T) S.prev[nx] = m;
-            P.alive[at(P, n, p)] = 0;
-            S.sim[n] = -INFINITY;
-        }
-        __syncthreads();
-        // ---- similarities on both sides of every changed row
-        const int nch = s_cnt;
-        for (int task = warp; task < 2 * nch; task += kMlWarps) {
-            const int j = nxt[task >> 1];
-            int a, b;
-            if (task & 1) { a = j; b = S.next[j]; }
-            else { a = S.prev[j]; b = j; }
-            if (a < 0) continue;
-            float sv = -INFINITY;
-            if (b < T) sv = warp_pair_sim(row(a), S.nrm[a], row(b), S.nrm[b], C, lane);
-            if (lane == 0) S.sim[a] = sv;
-        }
-        nd = nch;
-        __syncthreads();
-    }
+    __nv_bfloat16* rowbuf = reinterpret_cast<__nv_bfloat16*>(smem_raw + L.rowbuf);
+    for (int r = 0; r < rounds; ++r) mallm_round<kBufs>(P, c, rowbuf, r, block_argmax(c.sim_, 1, T, s_best));
 }
 
 // ------------------------------------------------------------------------------------- sync mode: mean + argmax
@@ -584,6 +502,36 @@ __device__ __forceinline__ float aten_row_sum_bf16(const float* __restrict__ row
     return s;
 }
 
+// Block-wide exclusive count of the surviving frames of patch p.  Each thread owns one chunk [i0, i1) of
+// ceil(T / blockDim.x) frames, in thread order; the result is the number of survivors before i0.  `warp_tot`: 32 ints.
+__device__ __forceinline__ int alive_before(const MallmParams& P, int p, int& i0, int& i1, int* warp_tot) {
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
+    const int per = (P.T + blockDim.x - 1) / blockDim.x;
+    i0 = threadIdx.x * per;
+    i1 = min(P.T, i0 + per);
+    int cnt = 0;
+    for (int i = i0; i < i1; ++i) cnt += P.alive[at(P, i, p)];
+    int inc = cnt;
+#pragma unroll
+    for (int off = 1; off < 32; off <<= 1) {
+        const int o = __shfl_up_sync(0xffffffffu, inc, off);
+        if (lane >= off) inc += o;
+    }
+    if (lane == 31) warp_tot[warp] = inc;
+    __syncthreads();
+    if (warp == 0) {
+        int t = (lane < nw) ? warp_tot[lane] : 0;
+#pragma unroll
+        for (int off = 1; off < 32; off <<= 1) {
+            const int o = __shfl_up_sync(0xffffffffu, t, off);
+            if (lane >= off) t += o;
+        }
+        warp_tot[lane] = t;
+    }
+    __syncthreads();
+    return inc - cnt + (warp ? warp_tot[warp - 1] : 0);
+}
+
 // one CTA: refresh the mean similarity of the rows rewritten in the round stamped `stamp` (all rows when the row
 // alignment depends on the position, i.e. N % 8 != 0), then the shared argmax
 __global__ void __launch_bounds__(1024) mallm_sync_argmax_kernel(MallmParams P, int stamp) {
@@ -596,30 +544,8 @@ __global__ void __launch_bounds__(1024) mallm_sync_argmax_kernel(MallmParams P, 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, nw = blockDim.x >> 5;
     const bool all = (N & 7) != 0 || stamp == 0;
     if (all && N >= 128 && (N & 7)) {
-        // exclusive scan of the alive flags, chunk per thread
-        const int per = (T + blockDim.x - 1) / blockDim.x;
-        const int i0 = threadIdx.x * per, i1 = min(T, i0 + per);
-        int cnt = 0;
-        for (int i = i0; i < i1; ++i) cnt += P.alive[at(P, i, 0)];
-        int inc = cnt;
-#pragma unroll
-        for (int off = 1; off < 32; off <<= 1) {
-            const int o = __shfl_up_sync(0xffffffffu, inc, off);
-            if (lane >= off) inc += o;
-        }
-        if (lane == 31) s_warp_tot[warp] = inc;
-        __syncthreads();
-        if (warp == 0) {
-            int t = (lane < nw) ? s_warp_tot[lane] : 0;
-#pragma unroll
-            for (int off = 1; off < 32; off <<= 1) {
-                const int o = __shfl_up_sync(0xffffffffu, t, off);
-                if (lane >= off) t += o;
-            }
-            s_warp_tot[lane] = t;
-        }
-        __syncthreads();
-        int run = inc - cnt + (warp ? s_warp_tot[warp - 1] : 0);
+        int i0, i1;
+        int run = alive_before(P, 0, i0, i1, s_warp_tot);
         for (int i = i0; i < i1; ++i) {
             pos[i] = run;
             run += P.alive[at(P, i, 0)];
@@ -659,23 +585,11 @@ __global__ void __launch_bounds__(kMlThreads) mallm_emit_kernel(MallmParams P, _
     pdl_enter();
     extern __shared__ __align__(16) uint8_t smem_raw[];
     int* order = reinterpret_cast<int*>(smem_raw);               // [t]
-    __shared__ int s_warp_tot[kMlWarps];
+    __shared__ int s_warp_tot[32];
     const int p = blockIdx.x, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const int T = P.T;
-    const int per = (T + kMlThreads - 1) / kMlThreads;
-    const int i0 = threadIdx.x * per, i1 = min(T, i0 + per);
-    int cnt = 0;
-    for (int i = i0; i < i1; ++i) cnt += P.alive[at(P, i, p)];
-    int inc = cnt;
-#pragma unroll
-    for (int off = 1; off < 32; off <<= 1) {
-        const int o = __shfl_up_sync(0xffffffffu, inc, off);
-        if (lane >= off) inc += o;
-    }
-    if (lane == 31) s_warp_tot[warp] = inc;
-    __syncthreads();
-    int base = inc - cnt;
-    for (int w = 0; w < warp; ++w) base += s_warp_tot[w];
+    const GlobalColumn c(P, p);
+    int i0, i1;
+    int base = alive_before(P, p, i0, i1, s_warp_tot);
     for (int i = i0; i < i1; ++i)
         if (P.alive[at(P, i, p)]) {
             if (base < t) order[base] = i;
@@ -685,7 +599,7 @@ __global__ void __launch_bounds__(kMlThreads) mallm_emit_kernel(MallmParams P, _
     const int nvec = P.C >> 3;
     for (int j = warp; j < t; j += kMlWarps) {
         const int i = order[j];
-        const uint4* src = reinterpret_cast<const uint4*>(row_ptr(P, i, p));
+        const uint4* src = reinterpret_cast<const uint4*>(c.row(i));
         uint4* dst = reinterpret_cast<uint4*>(out + ((size_t)j * P.N + p) * (size_t)P.C);
         int v = lane;
         for (; v + (kBatch - 1) * 32 < nvec; v += kBatch * 32) {
@@ -696,7 +610,7 @@ __global__ void __launch_bounds__(kMlThreads) mallm_emit_kernel(MallmParams P, _
             for (int u = 0; u < kBatch; ++u) dst[v + 32 * u] = b[u];
         }
         for (; v < nvec; v += 32) dst[v] = src[v];
-        if (lane == 0 && sizes_out) sizes_out[(size_t)j * P.N + p] = __float2bfloat16_rn(P.size[at(P, i, p)]);
+        if (lane == 0 && sizes_out) sizes_out[(size_t)j * P.N + p] = __float2bfloat16_rn(c.size(i));
     }
 }
 
@@ -768,46 +682,45 @@ extern "C" int rtk_mallm_compress(const void* x, const void* sizes_in, int64_t T
     P.touched = reinterpret_cast<int*>(ws + L.touched);
     P.sync = sync ? 1 : 0;
     P.hard = hard ? 1 : 0;
+    const int rounds = (int)(T - t);
     const size_t scan_smem = (size_t)T * 8;                     // positions + task list of the sync argmax kernel
-    if (sync) {
-        cudaError_t e = cudaFuncSetAttribute(mallm_sync_argmax_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)scan_smem);
+    const size_t row_smem = hard ? 0 : (size_t)kSyncBufs * C * 2;   // row buffers of the sync round kernel, <= 32 KB
+    const size_t emit_smem = (size_t)t * 4;
+    void (*rounds_kernel)(MallmParams, int) = mallm_rounds_kernel<2>;
+    size_t rounds_bytes = 0;
+    cudaError_t e;
+    if (!sync && rounds > 0) {
+        // the per-patch state in shared memory, with two row buffers when they fit (1 KB is left for the kernel's
+        // static shared memory); one buffer fits up to T = C = 8192 on a B200
+        int dev = 0, optin = 0;
+        if ((e = cudaGetDevice(&dev)) != cudaSuccess) return (int)e;
+        if ((e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev)) != cudaSuccess) return (int)e;
+        const int bufs = rounds_smem((int)T, (int)C, 2).bytes + 1024 <= (size_t)optin ? 2 : 1;
+        rounds_bytes = rounds_smem((int)T, (int)C, bufs).bytes;
+        if (rounds_bytes + 1024 > (size_t)optin) return RTK_E_UNSUPPORTED;
+        if (bufs == 1) rounds_kernel = mallm_rounds_kernel<1>;
+        e = cudaFuncSetAttribute(rounds_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)rounds_bytes);
         if (e != cudaSuccess) return (int)e;
     }
+    if (sync) {
+        e = cudaFuncSetAttribute(mallm_sync_argmax_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)scan_smem);
+        if (e != cudaSuccess) return (int)e;
+    }
+    e = cudaFuncSetAttribute(mallm_emit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)emit_smem);
+    if (e != cudaSuccess) return (int)e;
     if (T >= 2) {
         const int rc = dpselect_sim_nrm(x, T, N, C, DisAux{P.sim, P.nrm, P.si, P.sp}, stream);
         if (rc) return rc;
     }
     RTK_LAUNCH_PDL(mallm_init_kernel, (unsigned)N, kMlThreads, 0, stream, P);
-    if (sync && t < T) {
-        RTK_LAUNCH_PDL(mallm_sync_argmax_kernel, 1, 1024, scan_smem, stream, P, 0);
-    }
-    const int rounds = (int)(T - t);
     if (!sync) {
-        if (rounds > 0) {
-            int dev = 0, smem_max = 0;
-            cudaGetDevice(&dev);
-            cudaDeviceGetAttribute(&smem_max, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
-            const size_t need = rounds_smem_bytes((int)T, (int)C);
-            if (need + 1024 <= (size_t)smem_max) {                 // whole per-patch state in shared memory
-                cudaError_t e2 = cudaFuncSetAttribute(mallm_rounds_smem_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)need);
-                if (e2 != cudaSuccess) return (int)e2;
-                RTK_LAUNCH_PDL(mallm_rounds_smem_kernel, (unsigned)N, kMlThreads, need, stream, P, rounds);
-            } else {                                              // very long videos: state stays in global memory
-                // only the similarity column lives in shared memory: T floats, at most 32 KB, under the 48 KB default
-                RTK_LAUNCH_PDL(mallm_rounds_kernel, (unsigned)N, kMlThreads, (size_t)T * 4, stream, P, rounds);
-            }
-        }
+        if (rounds > 0) RTK_LAUNCH_PDL(rounds_kernel, (unsigned)N, kMlThreads, rounds_bytes, stream, P, rounds);
     } else {
         for (int r = 0; r < rounds; ++r) {
-            RTK_LAUNCH_PDL(mallm_round_kernel, (unsigned)N, kMlThreads, 0, stream, P, r);
-            if (r + 1 < rounds) {
-                RTK_LAUNCH_PDL(mallm_sync_argmax_kernel, 1, 1024, scan_smem, stream, P, r + 1);
-            }
+            RTK_LAUNCH_PDL(mallm_sync_argmax_kernel, 1, 1024, scan_smem, stream, P, r);
+            RTK_LAUNCH_PDL(mallm_round_kernel, (unsigned)N, kMlThreads, row_smem, stream, P, r);
         }
     }
-    const size_t emit_smem = (size_t)t * 4;
-    cudaError_t e = cudaFuncSetAttribute(mallm_emit_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)emit_smem);
-    if (e != cudaSuccess) return (int)e;
     RTK_LAUNCH_PDL(mallm_emit_kernel, (unsigned)N, kMlThreads, emit_smem, stream, P, static_cast<__nv_bfloat16*>(out), hard ? nullptr : static_cast<__nv_bfloat16*>(sizes_out), (int)t);
     return 0;
 }
