@@ -73,6 +73,9 @@ int rtk_dpselect_dis(const void* x, int64_t T, int64_t N, int64_t C, int halo, f
  *   t      1 <= t <= T
  *   idx    int32 [t, N] (sync=0) or [t] (sync=1): kept frame index per output slot, ascending in dim 0
  *   mask   uint8 [t * N]: 1 where the kept (frame, patch) is a peak (row-major j * N + p)
+ * Peaks replay ATen's max-pool window loop: the window [i-1, i+1] (clipped to [0, T)) starts at its first position with
+ * max -inf and takes v when v > max || isnan(v); frame i is a peak when the loop ends on i.  On finite values that is
+ * the first maximum; a run of NaNs peaks at the last NaN of each window.
  * Ties at the t-th key are resolved like ATen's CUDA radix select: larger keys first, equal keys by
  * ascending frame index; key order is the radix order (-0 < +0, NaN largest).
  */

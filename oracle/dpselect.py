@@ -11,7 +11,7 @@ individual roundings are written out, so that the CUDA kernels have a spec:
 * ``max_pool1d_with_indices(window 3, stride 1, pad 1)`` + ``unique`` + ``nonzero``
   (``:121-123`` / ``:153-156``) selects frame i iff ``d[i] > d[i-1]`` (strict; no left
   neighbour for i = 0) and ``d[i] >= d[i+1]`` (no right neighbour for the last) - the
-  pool keeps the FIRST maximum of each window (note N2).
+  pool keeps the FIRST maximum of each window, but the LAST NaN (note N2, ``peak_mask``).
 * ``d[peaks] += 2`` in fp32, ``topk(k=t, sorted=False)`` then ascending index sort
   (``:133-135`` / ``:160,167-168``).  ``torch.topk`` leaves the choice among equal keys
   unspecified; the oracle offers the two rules that matter: ``tie="lowest"`` (all keys
@@ -101,14 +101,22 @@ def adjacent_cosine_distance(x: torch.Tensor, reduce: str = "torch", norm_vec: i
 
 
 def peak_mask(d: torch.Tensor) -> torch.Tensor:
-    """Boolean peaks along dim 0 of ``d[T, ...]``: strict rise on the left, no rise on the right."""
+    """Boolean peaks along dim 0 of ``d[T, ...]``: ATen's ``max_pool1d_with_indices(window 3, pad 1)`` loop, literally.
+    The window [i-1, i+1] (clipped to [0, T)) starts at its first position with max -inf and takes v when
+    ``v > max or isnan(v)``; i is a peak when the loop ends on i.  On finite values: strict rise on the left, no rise on
+    the right.  In a run of NaNs the LAST NaN of each window wins (note N2)."""
     T = d.shape[0]
-    left = torch.ones_like(d, dtype=torch.bool)
-    right = torch.ones_like(d, dtype=torch.bool)
-    if T > 1:
-        left[1:] = d[1:] > d[:-1]
-        right[:-1] = d[:-1] >= d[1:]
-    return left & right
+    pos = torch.arange(T, device=d.device).reshape((T,) + (1,) * (d.dim() - 1))
+    arg = (pos - 1).clamp_min(0).expand(d.shape)
+    mx = torch.full_like(d, float("-inf"))
+    for u in (-1, 0, 1):
+        j = pos + u
+        valid = (j >= 0) & (j < T)
+        v = d[(j.clamp(0, T - 1)).flatten()]
+        take = valid & ((v > mx) | torch.isnan(v))
+        mx = torch.where(take, v, mx)
+        arg = torch.where(take, j, arg)
+    return arg == pos
 
 
 def select_top(keys: torch.Tensor, t: int, tie: str = "lowest") -> torch.Tensor:

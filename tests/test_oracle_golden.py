@@ -80,6 +80,44 @@ def test_kat_d1_known_answers():
     assert od.memory_bank_compress_keyframe(x, 2, sync=True, return_indices=True)[2].tolist() == [0, 2]
 
 
+def _aten_peaks(rows):
+    """the reference's peak rule on rows [R, T] (visual_compression.py:121-123): max_pool1d_with_indices, CPU"""
+    import torch.nn.functional as F
+    arg = F.max_pool1d_with_indices(rows[:, None, :], 3, 1, padding=1)[1][:, 0]
+    return arg == torch.arange(rows.shape[1])[None]
+
+
+def test_peak_mask_equals_max_pool_on_nan_and_inf_patterns():
+    """oracle peak rule == ATen's max_pool1d_with_indices on every pattern of {NaN, +inf, -inf, 0, 1, 2} over 5 frames,
+    NaN runs of length 1-3 at the start, middle and end of long columns, and the sync layout (one row)"""
+    vals = torch.tensor([float("nan"), float("inf"), float("-inf"), 0.0, 1.0, 2.0])
+    T = 5
+    codes = torch.cartesian_prod(*[torch.arange(len(vals))] * T)                     # [6^5, 5]
+    rows = vals[codes]
+    want = _aten_peaks(rows)
+    assert torch.equal(od.peak_mask(rows.t().contiguous()).t(), want)
+    for r in range(0, rows.shape[0], 997):                                            # the 1-D (sync) form
+        assert torch.equal(od.peak_mask(rows[r]), want[r])
+    g = torch.Generator().manual_seed(8)
+    cols = []
+    for run in (1, 2, 3):
+        for at in (0, 20, 40 - run):
+            c = torch.rand(40, generator=g)
+            c[at:at + run] = float("nan")
+            cols.append(c)
+    for fill in (float("inf"), float("-inf")):
+        c = torch.rand(40, generator=g)
+        c[5:8] = fill
+        c[30:32] = fill
+        cols.append(c)
+    rows = torch.stack(cols)
+    assert torch.equal(od.peak_mask(rows.t()).t(), _aten_peaks(rows))
+    # the pattern of one bad bank element: two adjacent NaN distances; the second one is the peak
+    d = torch.tensor([1.0, .95, .96, .97, .95, float("nan"), float("nan"), .95, 1.04, 1.0])
+    assert torch.nonzero(od.peak_mask(d))[:, 0].tolist() == [0, 3, 6, 8]
+    assert torch.equal(od.peak_mask(d), _aten_peaks(d[None])[0])
+
+
 def test_aten_cuda_rowsum_agrees_with_plain_sum():
     g = torch.Generator().manual_seed(3)
     x = torch.randn(64, 1152, generator=g)

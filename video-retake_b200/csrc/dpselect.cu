@@ -252,11 +252,22 @@ __device__ __forceinline__ void warp_select_top(const uint32_t* keys, int T, int
 }
 
 __device__ __forceinline__ bool is_peak(const float* d, int i, int T) {
-    // max_pool1d_with_indices(window 3, pad 1) keeps the first maximum: strict on the left, >= on the right
-    const float c = d[i];
-    const bool l = (i == 0) || (c > d[i - 1]) || (c != c && d[i - 1] == d[i - 1]);
-    const bool r = (i == T - 1) || (c >= d[i + 1]) || (c != c);
-    return l && r;
+    // ATen's max_pool1d_with_indices(window 3, pad 1) window loop, literally: the argmax starts at the window's first
+    // valid position with max -inf, and v is taken when v > max || isnan(v).  On finite values that keeps the first
+    // maximum (strict on the left, >= on the right); in a run of NaNs it keeps the LAST NaN of the window.
+    int arg = max(i - 1, 0);
+    float mx = -INFINITY;
+#pragma unroll
+    for (int u = -1; u <= 1; ++u) {
+        const int j = i + u;
+        if (j < 0 || j >= T) continue;
+        const float v = d[j];
+        if (v > mx || v != v) {
+            mx = v;
+            arg = j;
+        }
+    }
+    return arg == i;
 }
 
 // sync == 0: a CTA of W warps (W = blockDim.x / 32, a power of two <= 8) handles W consecutive patch columns, one warp
